@@ -34,6 +34,7 @@ EXTRA = (0.0, 0.5, 0.0)
 FS = 24000
 THRESHOLD_DB = 60.0
 METRIC = 'chunks_per_s_0.3s_24kHz_encode_stage1_stage2_vocode'
+DUMP_BYTES = 64 << 20          # --dump-outputs: at most this much in all, over every rank and stream
 WORKLOAD = ('single stream per GPU, buffer_time=0.3 s, extras (0,0.5,0), frame_period 5 ms, 24 kHz in/out, '
             'convert window 260 -> 384 frames, stage-1 1-D U-Net base 64 (13.6 M params), '
             'stage-2 2-D U-Net base 64 on 384x512 (54.4 M params, 142 GFLOP/chunk), WORLD DIO+StoneMask/CheapTrick/D4C + realtime synthesis')
@@ -297,7 +298,7 @@ def run_gpu(args):
         Tw = round((T + 2 * EXTRA[1]) * 200)
         return Tw, Tw + (128 - Tw % 128)
 
-    def run_config(T, B, steps, warmup, with_e2e, sustain_s=0.0, f0_method='dio'):
+    def run_config(T, B, steps, warmup, with_e2e, sustain_s=0.0, f0_method='dio', dump_dir=None):
         """One workload (buffer_time T, B grouped streams per GPU) on every rank: device-resident leg, optional sustained repeat of
         the same K-step block, optional end-to-end leg with host buffers.  Returns a dict of rank-0 figures (times max over ranks)."""
         Tw, Tp = window(T)
@@ -364,6 +365,15 @@ def run_gpu(args):
         s2_sum, s2_ms, s2_runs = eng.profile_read2()   # s2_ms = union of the per-forward intervals (consecutive forwards overlap on two streams)
         eng.profile(False)
         clocks = sampler.stop()
+        if dump_dir is not None:
+            # the waveform every stream's caller received from the last timed push, read before the sustained leg reuses the ring slots;
+            # a stream whose share of DUMP_BYTES it would exceed is written as every k-th sample, the smallest k that fits
+            r = (total - 1) % RING
+            counts = d_n[r].cpu().numpy()
+            cap = max(1, DUMP_BYTES // (8 * world * B))
+            for j in range(B):
+                wave = d_out[r, j, :int(counts[j])].cpu().numpy().astype(np.float64)
+                np.save(dump_dir / f'wave_rank{rank}_stream{j}.npy', wave[::-(-len(wave) // cap)] if len(wave) > cap else wave)
         launches = eng.launch_count - launches0
         res = dict(T=T, B=B, Tw=Tw, Tp=Tp, n=n, t_dev=max_over_ranks(t_dev), t_host=t_host, s2_ms=s2_ms, s2_sum=s2_sum, s2_runs=s2_runs, launches=launches, clocks=clocks)
 
@@ -431,7 +441,11 @@ def run_gpu(args):
 
     T, B = args.buffer_time, args.streams_per_gpu
     default_workload = (B == 1 and abs(T - BUFFER_TIME) < 1e-9)
-    main = run_config(T, B, args.steps, args.warmup, with_e2e=True, sustain_s=(args.sustain if default_workload else 0.0))
+    dump_dir = None
+    if args.dump_outputs:
+        dump_dir = Path(args.dump_outputs)
+        dump_dir.mkdir(parents=True, exist_ok=True)
+    main = run_config(T, B, args.steps, args.warmup, with_e2e=True, sustain_s=(args.sustain if default_workload else 0.0), dump_dir=dump_dir)
     extras = []
     if default_workload and not args.no_extra:
         # BASELINE configs 3 and 5, short device-resident legs so that the driver's N = 1..8 runs record them too
@@ -530,7 +544,13 @@ def main():
     ap.add_argument('--buffer-time', type=float, default=BUFFER_TIME, help='seconds per chunk (default workload: 0.3)')
     ap.add_argument('--sustain', type=float, default=2.0, help='seconds of back-to-back K-step blocks for the `sustained` key (0 = skip)')
     ap.add_argument('--no-extra', action='store_true', help='skip the short BASELINE config 3 / 5 legs (`extra_configs`)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the float64 waveform each stream produced in the last timed step as '
+                         'DIR/wave_rank<r>_stream<j>.npy, at most 64 MB in all (a longer wave is written as every k-th sample); '
+                         'inputs and weights are seeded: equal arguments give equal inputs')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes what the timed GPU path computed; it applies to --impl b200 only')
     if args.steps is None:
         args.steps = 20 if args.impl == 'b200' else 6
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup

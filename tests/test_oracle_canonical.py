@@ -11,14 +11,14 @@ turns the self-inflicted part of the gap into numbers (quoted in DESIGN.md secti
 from pathlib import Path
 
 import numpy as np
-import pytest
 
 from oracle import pipeline as opipe
 from oracle import world as W
 from realtime_yukarin_b200 import synthetic
 
 CFG = opipe.PathConfig()
-AUDIO_A = Path('/root/reference/tests/data/audioA.wav')        # the reference's own fixture; read in place when the checkout is present
+# the reference's own recording tests/data/audioA.wav: its first 4 s at 24 kHz (tests/golden/make_reference_fixtures.py)
+AUDIO_A = Path(__file__).resolve().parent / 'golden' / 'audioA_24k_4s.wav'
 
 
 def _resynth(feat, canonical, chunk=60, skip=0):
@@ -71,7 +71,6 @@ def test_decide_10_11_on_synthetic_speech():
     assert r['shifted'] < 1e-12 * max(1.0, r[3][3])
 
 
-@pytest.mark.skipif(not AUDIO_A.exists(), reason='reference checkout (tests/data/audioA.wav) not present on this machine')
 def test_decide_10_11_on_the_reference_recording():
     from realtime_yukarin_b200 import wave_io
     import scipy.signal

@@ -103,10 +103,10 @@ def test_harvest_golden_fixture():
     assert np.allclose(f0, g['f0'], rtol=1e-9, atol=0)
 
 
-AUDIO_A = Path('/root/reference/tests/data/audioA.wav')        # the reference's own fixture; read in place when the checkout is present
+# the reference's own recording tests/data/audioA.wav: its first 4 s at 24 kHz (tests/golden/make_reference_fixtures.py)
+AUDIO_A = Path(__file__).resolve().parent / 'golden' / 'audioA_24k_4s.wav'
 
 
-@pytest.mark.skipif(not AUDIO_A.exists(), reason='reference checkout (tests/data/audioA.wav) not present on this machine')
 def test_harvest_on_the_reference_recording():
     """Real speech (the reference's tests/data/audioA.wav at 24 kHz, 4 s): Harvest and DIO + StoneMask -- two different published
     extractors restated independently of each other -- agree on the pitch where both are voiced, Harvest's contour is the smoother
