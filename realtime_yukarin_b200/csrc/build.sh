@@ -6,7 +6,7 @@ NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -Wno-unused-variable --expt-relaxed-constexpr $RYK_NVCC_EXTRA"
 OBJ=${RYK_OBJ_DIR:-_obj}
 mkdir -p $OBJ
-SRCS="api crepe conv_direct conv_tc conv_tc2 conv_tc3 s1_fused unet world_analysis world_harvest world_synth features convert session"
+SRCS="api crepe conv_direct conv_tc conv_tc3 s1_fused unet world_analysis world_harvest world_synth features convert session"
 pids=""
 for s in $SRCS; do
   if [ ! -f $OBJ/$s.o ] || [ $s.cu -nt $OBJ/$s.o ] || [ -n "$(find . -maxdepth 1 \( -name '*.h' -o -name '*.cuh' \) -newer $OBJ/$s.o 2>/dev/null)" ] || [ ../../include/ryk.h -nt $OBJ/$s.o ]; then

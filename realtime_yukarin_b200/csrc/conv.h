@@ -36,11 +36,8 @@ struct ConvLayer {
   int tile_w = 0, tile_h = 0;             // pixel tile = tile_w x tile_h = 128
   int block_n = 0;
   bool tc_ready = false;
-  // CTA-pair kernel (conv_tc2.cu): accumulator groups per pair (1 / 2 / 4 parity classes), N per group, half-tile weight map
-  bool tc2 = false; int tc2_groups = 0, tc2_ng = 0;
-  CUtensorMap tmB2;
   // halo kernel (conv_tc3.cu): persistent, dynamically scheduled; tile = t3_mt stacked M tiles of t3_tile_w x t3_tile_h pixels
-  bool tc3 = false; int t3_tile_w = 0, t3_tile_h = 0, t3_mt = 0; bool t3_one = false;   // t3_one: one tile per CTA, two CTAs per SM
+  bool tc3 = false; int t3_tile_w = 0, t3_tile_h = 0, t3_mt = 0;
   int* t3_ctr = nullptr;                   // tile counter (one zero-initialised int, owned by the plan; re-armed by the kernel itself)
   CUtensorMap t3A0, t3A1, t3B, t3O;
 };
@@ -57,7 +54,6 @@ int tc_init();                                           // resolves cuTensorMap
 int tc_layer_prepare(ConvLayer& L, int num_sms);         // builds tensor maps, picks tiles / split-K (needs final pointers)
 int conv_tc_run(const ConvLayer& L, cudaStream_t st);
 size_t tc_splitk_ws_bytes(const ConvLayer& L, int num_sms);
-bool tc_layer_clusterk(const ConvLayer& L);                 // split-K layer whose partial sums are reduced inside the kernel (no reduce launch)
 void tc_force_pdl(int v);                                // -1 environment default, 0 / 1 forced
 
 // s1_fused.cu: the whole 1-D U-Net as one cluster kernel
@@ -65,15 +61,9 @@ int s1_pack_weights(const float* d_w_chainer, int transposed, int Cin, int Cout,
 int s1_fused_init();
 int s1_fused_cluster_size();                             // CTAs of the cluster the kernel runs on (<= 0: unavailable)
 
-// conv_tc2.cu
-int tc2_init();
-bool tc2_layer_config(const ConvLayer& L, int num_sms, int* groups, int* ng);     // needs L.tile_w / tile_h
-int tc2_layer_prepare(ConvLayer& L, PFN_cuTensorMapEncodeTiled_v12000 encode);
-int conv_tc2_run(const ConvLayer& L, cudaStream_t st, bool pdl);
-
 // conv_tc3.cu
 int tc3_init();
-bool tc3_layer_config(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h, int* mt, bool* one);
+bool tc3_layer_config(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h, int* mt);
 int tc3_layer_prepare(ConvLayer& L, PFN_cuTensorMapEncodeTiled_v12000 encode);     // needs L.t3_ctr
 int conv_tc3_run(const ConvLayer& L, cudaStream_t st, bool pdl);
 bool tc_layer_wants_counter(const ConvLayer& L, int num_sms);                         // true: allocate L.t3_ctr before tc_layer_prepare

@@ -18,8 +18,8 @@
 //     warps 0-3     : epilogue            (wait tmem_full, tcgen05.ld 32 lanes x 32 columns at a time,
 //                                          folded BN scale/shift + LeakyReLU/ReLU, FP16 NHWC store)
 // * Small-M bottleneck layers are weight-bandwidth bound: split-K over blockIdx.z spreads the weight
-//   stream over all SMs, partial sums meet in an FP32 workspace (red.global.add) and a finalize
-//   kernel applies the epilogue.
+//   stream over all SMs; each split stores its FP32 partial tile into its own slice of a workspace,
+//   and a reduce kernel sums the slices in a fixed order (deterministic) and applies the epilogue.
 #include <cuda.h>
 #include <cudaTypedefs.h>
 #include <stdlib.h>
@@ -32,8 +32,7 @@
 namespace ryk {
 
 struct TcParams {
-  int transposed, B, Hout, Wout, Cout;
-  int Hc, Wc;                    // class-local output grid (== Hout, Wout for convs)
+  int transposed, Cout;
   int tile_w, tile_h, tiles_w, tiles_h;
   int chunks0, chunks1;          // 64-channel chunks of source 0 / 1
   int taps_w, ntaps;             // taps per class: conv KH*KW (taps_w = KW); deconv (KH/SH)*(KW/SW)
@@ -42,16 +41,12 @@ struct TcParams {
   int ksplit, chunks_per_split;
   int act;
   const float* scale; const float* shift;
-  __half* out;
   float* ws;                     // split-K workspace [ksplit][pixels][Cout] or nullptr
-  size_t out_pixels;             // B * Hout * Wout
   int debug;                     // RYK_TC_DEBUG bit 1 (perf experiments only): skip the output stores
-  int cluster_k;                 // split-K partial sums are reduced INSIDE the kernel: the ksplit CTAs of a tile form a thread-block cluster
-                                 // (cluster rank == split) and read each other's FP32 partial tiles through distributed shared memory
 };
 
 #ifdef RYK_TC_TIMELINE
-// diagnostics build only (RYK_NVCC_EXTRA=-DRYK_TC_TIMELINE): per-CTA phase timestamps of the non-persistent kernel
+// diagnostics build only (RYK_NVCC_EXTRA=-DRYK_TC_TIMELINE): per-CTA phase timestamps
 constexpr int kTlMaxCtas = 8192, kTlSlots = 10;
 __device__ unsigned long long g_tl[kTlMaxCtas * kTlSlots];
 __device__ __forceinline__ unsigned long long tl_now() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
@@ -59,17 +54,15 @@ __device__ __forceinline__ unsigned long long tl_now() { unsigned long long t; a
 #else
 #define TL(slot) do {} while (0)
 #endif
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar);
-template <int BLOCK_N, int kStages, int kMinBlocks>
-__global__ void __launch_bounds__(kTcThreads, kMinBlocks)
+// Two co-resident CTAs per SM let one tile's epilogue overlap the other's main loop.
+template <int BLOCK_N, int kStages>
+__global__ void __launch_bounds__(kTcThreads, 2)
 k_conv_tc(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
           const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmW,
           const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   constexpr uint32_t kABytes = kBlockM * kBlockK * 2;
   constexpr uint32_t kBBytes = BLOCK_N * kBlockK * 2;
-  constexpr uint32_t kCkPitch = BLOCK_N * 4 + 16;          // row pitch of the FP32 partial tile of the in-cluster split-K reduction
-  constexpr bool kCkOk = (size_t)kBlockM * kCkPitch <= (size_t)kStages * (kABytes + kBBytes);      // partial tile fits the stage buffers (host side: variant 1 only)
   // carve: 1024-aligned stage buffers first, barriers after
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* smem_a = smem;
@@ -202,47 +195,40 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUte
             "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
           : "r"(taddr));
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      {
-        if (kCkOk && p.cluster_k) {
-          // raw FP32 partial sums -> plain [pixel][channel] tile in the (idle) stage buffers, row pitch kCkPitch; the cluster reduces below
-          uint8_t* dst = smem + (size_t)row * kCkPitch + c0 * 4;
+      if (p.ws) {
+        // split-K partial tile (raw FP32 sums) -> swizzled staging, one [128 pixels][32 channels] block per iteration;
+        // stored below by TMA into this split's slice of the workspace; k_splitk_reduce sums the slices
+        uint8_t* blk = smem + (c0 >> 5) * (kBlockM * 128) + row * 128;
 #pragma unroll
-          for (int j = 0; j < 8; ++j) *reinterpret_cast<uint4*>(dst + j * 16) = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
-        } else if (p.ws) {
-          // split-K partial tile (raw FP32 sums) -> swizzled staging, one [128 pixels][32 channels] block per iteration;
-          // stored below by TMA into this split's slice of the workspace; k_splitk_reduce sums the slices
-          uint8_t* blk = smem + (c0 >> 5) * (kBlockM * 128) + row * 128;
+        for (int j = 0; j < 8; ++j)
+          *reinterpret_cast<uint4*>(blk + ((j ^ (row & 7)) << 4)) = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
+      } else {
+        // scale/shift/activation -> FP16 -> 128B-swizzled staging tile in the (now idle) pipeline stage buffers:
+        // BLOCK_N / 64 blocks of [128 pixels][64 channels]; one TMA store per block writes full 128-byte rows
+        uint8_t* blk = smem + (c0 >> 6) * (kBlockM * 128) + row * 128;
+        const int cbase = (c0 & 32) >> 3;          // first 16-byte chunk of this 32-channel half inside the block: 0 or 4
 #pragma unroll
-          for (int j = 0; j < 8; ++j)
-            *reinterpret_cast<uint4*>(blk + ((j ^ (row & 7)) << 4)) = make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
-        } else {
-          // scale/shift/activation -> FP16 -> 128B-swizzled staging tile in the (now idle) pipeline stage buffers:
-          // BLOCK_N / 64 blocks of [128 pixels][64 channels]; one TMA store per block writes full 128-byte rows
-          uint8_t* blk = smem + (c0 >> 6) * (kBlockM * 128) + row * 128;
-          const int cbase = (c0 & 32) >> 3;          // first 16-byte chunk of this 32-channel half inside the block: 0 or 4
+        for (int j = 0; j < 32; j += 8) {
+          const float4 sc0 = *reinterpret_cast<const float4*>(s_scale + c0 + j), sc1 = *reinterpret_cast<const float4*>(s_scale + c0 + j + 4);
+          const float4 sh0 = *reinterpret_cast<const float4*>(s_shift + c0 + j), sh1 = *reinterpret_cast<const float4*>(s_shift + c0 + j + 4);
+          const float sc[8] = {sc0.x, sc0.y, sc0.z, sc0.w, sc1.x, sc1.y, sc1.z, sc1.w};
+          const float sh[8] = {sh0.x, sh0.y, sh0.z, sh0.w, sh1.x, sh1.y, sh1.z, sh1.w};
+          uint32_t pk[4];
 #pragma unroll
-          for (int j = 0; j < 32; j += 8) {
-            const float4 sc0 = *reinterpret_cast<const float4*>(s_scale + c0 + j), sc1 = *reinterpret_cast<const float4*>(s_scale + c0 + j + 4);
-            const float4 sh0 = *reinterpret_cast<const float4*>(s_shift + c0 + j), sh1 = *reinterpret_cast<const float4*>(s_shift + c0 + j + 4);
-            const float sc[8] = {sc0.x, sc0.y, sc0.z, sc0.w, sc1.x, sc1.y, sc1.z, sc1.w};
-            const float sh[8] = {sh0.x, sh0.y, sh0.z, sh0.w, sh1.x, sh1.y, sh1.z, sh1.w};
-            uint32_t pk[4];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              float v0 = fmaf(__uint_as_float(r[j + 2 * q]), sc[2 * q], sh[2 * q]);
-              float v1 = fmaf(__uint_as_float(r[j + 2 * q + 1]), sc[2 * q + 1], sh[2 * q + 1]);
-              if (p.act == ACT_LEAKY) { v0 = v0 > 0.f ? v0 : 0.2f * v0; v1 = v1 > 0.f ? v1 : 0.2f * v1; }
-              else if (p.act == ACT_RELU) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); }
-              __half2 h = __floats2half2_rn(v0, v1);
-              pk[q] = *reinterpret_cast<uint32_t*>(&h);
-            }
-            const int chunk = cbase + (j >> 3);
-            *reinterpret_cast<uint4*>(blk + ((chunk ^ (row & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+          for (int q = 0; q < 4; ++q) {
+            float v0 = fmaf(__uint_as_float(r[j + 2 * q]), sc[2 * q], sh[2 * q]);
+            float v1 = fmaf(__uint_as_float(r[j + 2 * q + 1]), sc[2 * q + 1], sh[2 * q + 1]);
+            if (p.act == ACT_LEAKY) { v0 = v0 > 0.f ? v0 : 0.2f * v0; v1 = v1 > 0.f ? v1 : 0.2f * v1; }
+            else if (p.act == ACT_RELU) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); }
+            __half2 h = __floats2half2_rn(v0, v1);
+            pk[q] = *reinterpret_cast<uint32_t*>(&h);
           }
+          const int chunk = cbase + (j >> 3);
+          *reinterpret_cast<uint4*>(blk + ((chunk ^ (row & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         }
       }
     }
-    if (!p.ws && !p.cluster_k && my_chunks > 0) {
+    if (!p.ws && my_chunks > 0) {
       // generic-proxy smem writes -> visible to the async proxy; one thread hands the tile to the TMA unit
       // (out-of-range pixels are clipped by the tensor map, so no masking is needed)
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -275,291 +261,12 @@ k_conv_tc(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUte
       }
     }
   }
-  if (kCkOk && p.cluster_k) {
-    // ===== in-cluster split-K reduction (replaces the FP32 workspace round trip + k_splitk_reduce launch) =====
-    // CTA r of the cluster (= split r) owns tile rows r, r + ksplit, ...; it sums the ksplit partial rows in split order (fixed:
-    // deterministic), applies scale / shift / activation and writes FP16 NHWC directly.  All threads take both cluster barriers.
-    cluster_barrier();                                   // every split's partial tile is in its CTA's shared memory
-    if (warp < 4) {
-      constexpr int kTpr = BLOCK_N / 4;                  // threads per row (one float4 each)
-      constexpr int kRpp = 128 / kTpr;                   // rows per pass
-      const int sub = threadIdx.x / kTpr, c4 = threadIdx.x % kTpr;
-      const uint32_t my_base = smem_u32(smem);
-      const float4 sc = *reinterpret_cast<const float4*>(s_scale + c4 * 4), sh = *reinterpret_cast<const float4*>(s_shift + c4 * 4);
-      for (int i = sub; ; i += kRpp) {
-        const int row = split + i * p.ksplit;
-        if (row >= kBlockM) break;
-        const int hl = row / p.tile_w, wl = row - hl * p.tile_w;
-        const int my = oy0 + hl, mx = ox0 + wl;
-        if (my >= p.Hc || mx >= p.Wc) continue;
-        const uint32_t off = (uint32_t)row * kCkPitch + (uint32_t)c4 * 16u;
-        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int q = 0; q < p.ksplit; ++q) {
-          const float4 v = ld_cluster_f4(cluster_map_rank(my_base + off, (uint32_t)q));
-          a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
-        }
-        float v4[4] = {fmaf(a.x, sc.x, sh.x), fmaf(a.y, sc.y, sh.y), fmaf(a.z, sc.z, sh.z), fmaf(a.w, sc.w, sh.w)};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if (p.act == ACT_LEAKY) v4[j] = v4[j] > 0.f ? v4[j] : 0.2f * v4[j]; else if (p.act == ACT_RELU) v4[j] = fmaxf(v4[j], 0.f);
-        }
-        const int oy = p.transposed ? my * p.sh + py : my, ox = p.transposed ? mx * p.sw + px : mx;
-        __half2 h0 = __floats2half2_rn(v4[0], v4[1]), h1 = __floats2half2_rn(v4[2], v4[3]);
-        __half* dst = p.out + ((size_t)(b * p.Hout + oy) * p.Wout + ox) * p.Cout + n0 + c4 * 4;
-        *reinterpret_cast<uint2*>(dst) = make_uint2(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1));
-      }
-    }
-    cluster_barrier();                                   // nobody exits (and frees its shared memory) while a peer may still read it
-  }
   if (threadIdx.x == 0) TL(5);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   if (warp == 4) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)BLOCK_N) : "memory");
     if (lane == 0) TL(6);
-  }
-}
-
-// ------------------------------------------------------------------------------------ persistent variant
-// One CTA per SM loops over output tiles (tile = blockIdx.x + i * gridDim.x).  The smem ring keeps streaming across
-// tile boundaries and the accumulator is double-buffered in TMEM (2 x BLOCK_N columns), so the epilogue of tile i
-// (tcgen05.ld -> scale/shift/act -> FP16 stores) overlaps the TMA + MMA main loop of tile i + 1, and the per-tile
-// fixed costs (TMEM alloc, barrier init, tensor-map fetch, pipeline fill) are paid once per CTA.
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-template <int BLOCK_N, int kStages, int MT>
-__global__ void __launch_bounds__(kTcThreads, 1)
-k_conv_tc_persist(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
-                  const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmO, const TcParams p,
-                  const int tiles_mn, const int n_tiles_n, const int total_tiles) {
-  // MT = pixel tiles (of 128) per CTA tile: MT = 2 makes a 256 x BLOCK_N CTA tile whose two halves share every B
-  // (weight) stage -- the k4 layers are bound by L2 -> shared-memory traffic (~10 TB/s), so bytes per FLOP matter.
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  constexpr uint32_t kAHalf = kBlockM * kBlockK * 2;
-  constexpr uint32_t kABytes = MT * kAHalf;
-  constexpr uint32_t kBBytes = BLOCK_N * kBlockK * 2;
-  constexpr int kAccStages = (2 * MT * BLOCK_N <= 512) ? 2 : 1;
-  constexpr uint32_t kTmemCols = kAccStages * MT * BLOCK_N;
-  uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint8_t* smem_a = smem;
-  uint8_t* smem_b = smem + kStages * kABytes;
-  // epilogue staging: BLOCK_N / 64 blocks of [128 pixels][64 channels] fp16 in the 128B-swizzled layout a TMA store reads
-  constexpr uint32_t kOutBytes = kBlockM * BLOCK_N * 2;
-  uint8_t* smem_out = smem_b + kStages * kBBytes;
-  uint64_t* full_bar = (uint64_t*)(smem_out + kOutBytes);
-  uint64_t* empty_bar = full_bar + kStages;
-  uint64_t* tfull_bar = empty_bar + kStages;      // [2]
-  uint64_t* tempty_bar = tfull_bar + 2;            // [2]
-  uint32_t* tmem_ptr_smem = (uint32_t*)(tempty_bar + 2);
-  float* s_scale = (float*)(((uintptr_t)(tmem_ptr_smem + 4) + 15) & ~(uintptr_t)15);    // scale / shift of the current tile's channels (see k_conv_tc)
-  float* s_shift = s_scale + BLOCK_N;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  if (threadIdx.x == 128) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA0) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
-    if (p.chunks1 > 0) asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA1) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmO) : "memory");
-  }
-  if (threadIdx.x == 160) {
-    for (int i = 0; i < kStages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 4) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_ptr_smem)), "r"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_ptr_smem;
-
-  const int chunks_per_tap = p.chunks0 + p.chunks1;
-  const int total_chunks = p.ntaps * chunks_per_tap;
-  const int super_mn = (tiles_mn + MT - 1) / MT;
-
-  // tile decode: t -> (first m-tile, n-tile, class, split); m fastest so that co-running CTAs share the same weight tiles in L2
-  auto decode = [&](int t, int& mt0, int& n0, int& cls, int& split) {
-    mt0 = (t % super_mn) * MT; t /= super_mn;
-    int nt = t % n_tiles_n; t /= n_tiles_n;
-    split = t % p.ksplit; cls = t / p.ksplit;
-    n0 = nt * BLOCK_N;
-  };
-  auto decode_m = [&](int mt, int& tw, int& th, int& b) {
-    tw = mt % p.tiles_w; mt /= p.tiles_w;
-    th = mt % p.tiles_h; b = mt / p.tiles_h;       // b >= B for the padding half of an odd tile count: TMA zero-fills, stores are masked
-  };
-
-  if (warp == 4 && lane == 0) {
-    // ===== TMA producer =====
-    int it = 0;                                    // global chunk counter across tiles -> stage / phase
-    for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-      int mt0, n0, cls, split;
-      decode(t, mt0, n0, cls, split);
-      const int py = cls / p.classes_w, px = cls % p.classes_w;
-      const int kc_begin = split * p.chunks_per_split;
-      const int kc_end = min(total_chunks, kc_begin + p.chunks_per_split);
-      for (int kc = kc_begin; kc < kc_end; ++kc, ++it) {
-        const int s = it % kStages;
-        const uint32_t ph = (it / kStages) & 1;
-        mbar_wait(&empty_bar[s], ph ^ 1);
-        const int tap = kc / chunks_per_tap;
-        const int cc = kc - tap * chunks_per_tap;
-        const int ty = tap / p.taps_w, tx = tap - ty * p.taps_w;
-        mbar_expect_tx(&full_bar[s], kABytes + kBBytes);
-#pragma unroll
-        for (int h = 0; h < MT; ++h) {
-          int tw, th, b;
-          decode_m(mt0 + h, tw, th, b);
-          const int oy0 = th * p.tile_h, ox0 = tw * p.tile_w;
-          int ix, iy;
-          if (!p.transposed) { ix = ox0 * p.sw + tx - p.pw; iy = oy0 * p.sh + ty - p.ph; }
-          else { ix = p.sw == 2 ? ox0 + tx - 1 + px : ox0; iy = p.sh == 2 ? oy0 + ty - 1 + py : oy0; }
-          if (cc < p.chunks0) tma_load_4d(smem_a + s * kABytes + h * kAHalf, &tmA0, &full_bar[s], cc * kBlockK, ix, iy, b);
-          else tma_load_4d(smem_a + s * kABytes + h * kAHalf, &tmA1, &full_bar[s], (cc - p.chunks0) * kBlockK, ix, iy, b);
-        }
-        tma_load_2d(smem_b + s * kBBytes, &tmB, &full_bar[s], kc * kBlockK, cls * p.Cout + n0);
-      }
-    }
-  } else if (warp == 5 && lane == 0) {
-    // ===== MMA issuer =====
-    constexpr uint32_t idesc = (1u << 4) | ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)(kBlockM >> 4) << 24);
-    int it = 0, ti = 0;
-    for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++ti) {
-      int mt0, n0, cls, split;
-      decode(t, mt0, n0, cls, split);
-      const int kc_begin = split * p.chunks_per_split;
-      const int kc_end = min(total_chunks, kc_begin + p.chunks_per_split);
-      const int as = ti % kAccStages;
-      const uint32_t aph = (ti / kAccStages) & 1;
-      mbar_wait(&tempty_bar[as], aph ^ 1);          // epilogue has drained this accumulator
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      for (int kc = kc_begin; kc < kc_end; ++kc, ++it) {
-        const int s = it % kStages;
-        const uint32_t ph = (it / kStages) & 1;
-        mbar_wait(&full_bar[s], ph);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint64_t bdesc = make_sw128_desc(smem_u32(smem_b + s * kBBytes));
-#pragma unroll
-        for (int h = 0; h < MT; ++h) {
-          const uint64_t adesc = make_sw128_desc(smem_u32(smem_a + s * kABytes + h * kAHalf));
-          const uint32_t tmem_d = tmem_base + (uint32_t)((as * MT + h) * BLOCK_N);
-#pragma unroll
-          for (int k = 0; k < kBlockK / kUmmaK; ++k)
-            umma_f16(tmem_d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kc > kc_begin || k > 0) ? 1u : 0u);
-        }
-        umma_commit(&empty_bar[s]);
-      }
-      umma_commit(&tfull_bar[as]);
-    }
-  } else if (warp < 4) {
-    // ===== epilogue =====
-    int ti = 0;
-    for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++ti) {
-      int mt0, n0, cls, split;
-      decode(t, mt0, n0, cls, split);
-      const int py = cls / p.classes_w, px = cls % p.classes_w;
-      const int as = ti % kAccStages;
-      const uint32_t aph = (ti / kAccStages) & 1;
-      mbar_wait(&tfull_bar[as], aph);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const int row = warp * 32 + lane;
-#pragma unroll 1
-      for (int h = 0; h < MT; ++h) {
-        int tw, th, b;
-        decode_m(mt0 + h, tw, th, b);
-        const int oy0 = th * p.tile_h, ox0 = tw * p.tile_w;
-        const int hl = row / p.tile_w, wl = row - hl * p.tile_w;
-        const int my = oy0 + hl, mx = ox0 + wl;
-        const bool valid = (my < p.Hc) && (mx < p.Wc) && (b < p.B) && !(p.debug & 1);
-        int oy = my, ox = mx;
-        if (p.transposed) { oy = my * p.sh + py; ox = mx * p.sw + px; }
-        const size_t pix = ((size_t)(b * p.Hout + oy) * p.Wout + ox);
-        if (!p.ws) {
-          // the previous TMA store must have finished reading the staging buffer before it is overwritten
-          if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          if (h == 0) for (int i = threadIdx.x; i < BLOCK_N; i += 128) { s_scale[i] = __ldg(p.scale + n0 + i); s_shift[i] = __ldg(p.shift + n0 + i); }
-          asm volatile("bar.sync 1, 128;" ::: "memory");
-        }
-#pragma unroll 1
-        for (int c0 = 0; c0 < BLOCK_N; c0 += 32) {
-          uint32_t r[32];
-          const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)((as * MT + h) * BLOCK_N + c0);
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-              "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-              "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-              : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-                "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-                "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-              : "r"(taddr));
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-          if (h == MT - 1 && c0 + 32 >= BLOCK_N) {   // accumulator fully read: hand it back to the MMA warp before the stores
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty_bar[as]);
-          }
-          const int n = n0 + c0;
-          if (p.ws) {
-            if (valid) {
-              float4* w = reinterpret_cast<float4*>(p.ws + ((size_t)split * p.out_pixels + pix) * p.Cout + n);
-#pragma unroll
-              for (int j = 0; j < 8; ++j)
-                w[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
-            }
-          } else {
-            // scale/shift/activation -> FP16 -> swizzled staging tile (row = pixel, 8 x 16-byte chunks per 64-channel block)
-            uint8_t* blk = smem_out + (c0 >> 6) * (kBlockM * 128) + row * 128;
-            const int cbase = (c0 & 32) >> 3;          // first 16-byte chunk of this 32-channel half inside the block: 0 or 4
-#pragma unroll
-            for (int j = 0; j < 32; j += 8) {
-              const float4 sc0 = *reinterpret_cast<const float4*>(s_scale + c0 + j), sc1 = *reinterpret_cast<const float4*>(s_scale + c0 + j + 4);
-              const float4 sh0 = *reinterpret_cast<const float4*>(s_shift + c0 + j), sh1 = *reinterpret_cast<const float4*>(s_shift + c0 + j + 4);
-              const float sc[8] = {sc0.x, sc0.y, sc0.z, sc0.w, sc1.x, sc1.y, sc1.z, sc1.w};
-              const float sh[8] = {sh0.x, sh0.y, sh0.z, sh0.w, sh1.x, sh1.y, sh1.z, sh1.w};
-              uint32_t pk[4];
-#pragma unroll
-              for (int q = 0; q < 4; ++q) {
-                float v0 = fmaf(__uint_as_float(r[j + 2 * q]), sc[2 * q], sh[2 * q]);
-                float v1 = fmaf(__uint_as_float(r[j + 2 * q + 1]), sc[2 * q + 1], sh[2 * q + 1]);
-                if (p.act == ACT_LEAKY) { v0 = v0 > 0.f ? v0 : 0.2f * v0; v1 = v1 > 0.f ? v1 : 0.2f * v1; }
-                else if (p.act == ACT_RELU) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); }
-                __half2 h2 = __floats2half2_rn(v0, v1);
-                pk[q] = *reinterpret_cast<uint32_t*>(&h2);
-              }
-              const int chunk = cbase + (j >> 3);
-              *reinterpret_cast<uint4*>(blk + ((chunk ^ (row & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            }
-          }
-        }
-        if (!p.ws) {
-          // generic-proxy smem writes -> visible to the async proxy, then one thread hands the tile to the TMA unit:
-          // coalesced 128-byte rows, out-of-range pixels clipped by the tensor map (no masking needed)
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          asm volatile("bar.sync 1, 128;" ::: "memory");
-          if (threadIdx.x == 0 && !(p.debug & 1)) {
-            const int xs = p.transposed ? ox0 * p.sw + px : ox0;
-            const int ys = p.transposed ? oy0 * p.sh + py : oy0;
-#pragma unroll
-            for (int jb = 0; jb < BLOCK_N / 64; ++jb) {
-              asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                           ::"l"(&tmO), "r"(smem_u32(smem_out + jb * (kBlockM * 128))), "r"(n0 + jb * 64), "r"(xs), "r"(ys), "r"(b) : "memory");
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
-        }
-      }
-    }
-    if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (warp == 4) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
   }
 }
 
@@ -632,17 +339,6 @@ template <int BN, int ST> static constexpr size_t tc_smem_bytes() {
   return (size_t)ST * (kBlockM * kBlockK * 2 + BN * kBlockK * 2) + (2 * ST + 1) * 8 + 16 + 1024 + 2 * BN * 4 + 32;
 }
 
-// kernel variants: (BLOCK_N, stages, CTAs/SM). Two co-resident CTAs let one tile's epilogue overlap the other's main loop.
-static int g_variant = -1;
-static int tc_variant() {
-  if (g_variant < 0) { const char* v = getenv("RYK_TC_VARIANT"); g_variant = v ? atoi(v) : 1; }
-  return g_variant;
-}
-
-template <int BN, int ST, int MT> static constexpr size_t tcp_smem_bytes() {
-  return (size_t)ST * (MT * kBlockM * kBlockK * 2 + BN * kBlockK * 2) + (size_t)kBlockM * BN * 2 + (2 * ST + 4) * 8 + 16 + 1024 + 2 * BN * 4 + 32;
-}
-
 int tc_init() {
   if (!g_encode) {
     void* fn = nullptr;
@@ -651,22 +347,9 @@ int tc_init() {
     RYK_CHECK(qres == cudaDriverEntryPointSuccess && fn != nullptr, "cuTensorMapEncodeTiled not available from the driver");
     g_encode = (PFN_cuTensorMapEncodeTiled_v12000)fn;
   }
-  if (tc2_init()) return -1;
   if (tc3_init()) return -1;
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<64, 6, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<64, 6>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<128, 6, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<128, 6>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<256, 4, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<256, 4>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<64, 4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<64, 4>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<128, 3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<128, 3>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<256, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<256, 2>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<128, 2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<128, 2>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<64, 3, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<64, 3>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<64, 8, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<64, 8, 1>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<128, 6, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<128, 6, 1>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<256, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<256, 3, 1>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<64, 5, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<64, 5, 2>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<128, 4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<128, 4, 2>()));
-  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc_persist<256, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tcp_smem_bytes<256, 2, 2>()));
+  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<128, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<128, 3>()));
+  RYK_CUDA(cudaFuncSetAttribute(k_conv_tc<64, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes<64, 4>()));
   return 0;
 }
 
@@ -679,17 +362,6 @@ bool tc_layer_eligible(const ConvLayer& L) {
   if (L.in_dtype != DT_F16 || L.out_dtype != DT_F16) return false;
   return true;
 }
-
-// RYK_TC_CLUSTERK: 1 = split-K layers reduce their partial sums inside the kernel (thread-block cluster + distributed shared memory),
-// 0 (default) = FP32 workspace + k_splitk_reduce launch.  Measured (profiles/r02_layer_bench_cluster_splitk.txt): the DSMEM reduction
-// costs as much as the separate reduce launch on the bottleneck layers (c5 11.2 vs 10.3 us, d1 10.3 vs 11.1) and almost doubles c3 / d3
-// (32.9 vs 18.0 us: 43 rows x 3 remote reads per CTA at ~20 B/clk of DSMEM bandwidth) -- kept as an opt-in.
-static bool tc_clusterk() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RYK_TC_CLUSTERK"); v = (e && atoi(e) != 0) ? 1 : 0; }
-  return v != 0 && tc_variant() == 1;
-}
-bool tc_layer_clusterk(const ConvLayer& L) { return tc_clusterk() && L.ksplit > 1 && !L.tc2 && !L.tc3 && L.block_n <= 128; }
 
 static int pow2_floor(int v) { int p = 1; while (p * 2 <= v) p *= 2; return p; }
 
@@ -731,46 +403,40 @@ static int make_weight_map(CUtensorMap* m, const void* ptr, size_t K, size_t row
   return 0;
 }
 
+constexpr int kMinChunksPerSplit = 8;                  // split-K: at least this many 64-channel K chunks per split
+
 static void tc_geometry(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h, int* block_n, int* ksplit) {
   int Wc = L.transposed ? L.Win : L.Wout;
   int Hc = L.transposed ? L.Hin : L.Hout;
   int tw = pow2_floor(Wc < kBlockM ? Wc : kBlockM);
   int th = kBlockM / tw;
-  int bn = L.Cout >= 256 ? 256 : (L.Cout >= 128 ? 128 : 64);
-  if ((tc_variant() == 1 || tc_variant() == 2 || tc_variant() == 6) && bn == 256) bn = 128;   // non-persistent 2-CTAs/SM kernels: N <= 128 tiles (the epilogue staging must fit the stage buffers)
-  if (tc_variant() == 4 && bn == 256) bn = 128;        // variant 4: persistent with N <= 128
+  int bn = L.Cout >= 128 ? 128 : 64;                    // N <= 128: the epilogue's staging tile must fit the stage buffers
   int classes = L.transposed ? L.SH * L.SW : 1;
-  int tiles_mn_ = L.B * ((Wc + tw - 1) / tw) * ((Hc + th - 1) / th);
-  if (tc_variant() == 5) tiles_mn_ = (tiles_mn_ + 1) / 2;       // variant 5: 256-pixel CTA tiles
-  int tiles = tiles_mn_ * (L.Cout / bn) * classes;
+  int tiles = L.B * ((Wc + tw - 1) / tw) * ((Hc + th - 1) / th) * (L.Cout / bn) * classes;
   int ntaps = L.transposed ? (L.KH / L.SH) * (L.KW / L.SW) : L.KH * L.KW;
   int total_chunks = ntaps * (L.C0 + L.C1) / kBlockK;
   int ks = 1;
-  int slots = num_sms * (tc_variant() == 6 ? 3 : ((tc_variant() == 0 || tc_variant() >= 3) ? 1 : 2));
+  const int slots = 2 * num_sms;                        // two co-resident CTAs per SM
   if (tiles < slots) {
     ks = slots / tiles;
-    static int min_chunks = -1;
-    if (min_chunks < 0) { const char* v = getenv("RYK_TC_MIN_CHUNKS"); min_chunks = v ? atoi(v) : 8; if (min_chunks < 1) min_chunks = 1; }
-    if (ks > total_chunks / min_chunks) ks = total_chunks / min_chunks;   // at least min_chunks chunks per split
+    if (ks > total_chunks / kMinChunksPerSplit) ks = total_chunks / kMinChunksPerSplit;
     if (ks < 1) ks = 1;
-    if (tc_clusterk() && ks > 8) ks = 8;                // in-cluster reduction: the splits of a tile form one (portable-size) cluster
     int cps = (total_chunks + ks - 1) / ks;
     ks = (total_chunks + cps - 1) / cps;                // every split owns at least one chunk
   }
-  { ConvLayer T = L; T.tile_w = tw; T.tile_h = th; int g_, n_; if (tc2_layer_config(T, num_sms, &g_, &n_)) ks = 1; }   // pair kernel: no split-K
-  { int a_, b_, c_; bool o_; if (tc3_layer_config(L, num_sms, &a_, &b_, &c_, &o_)) ks = 1; }                                             // halo kernel: no split-K
+  { int a_, b_, c_; if (tc3_layer_config(L, num_sms, &a_, &b_, &c_)) ks = 1; }     // halo kernel: no split-K
   *tile_w = tw; *tile_h = th; *block_n = bn; *ksplit = ks;
 }
 
 bool tc_layer_wants_counter(const ConvLayer& L, int num_sms) {
-  int a_, b_, c_; bool o_;
-  return tc_layer_eligible(L) && tc3_layer_config(L, num_sms, &a_, &b_, &c_, &o_);
+  int a_, b_, c_;
+  return tc_layer_eligible(L) && tc3_layer_config(L, num_sms, &a_, &b_, &c_);
 }
 
 size_t tc_splitk_ws_bytes(const ConvLayer& L, int num_sms) {
   int tw, th, bn, ks;
   tc_geometry(L, num_sms, &tw, &th, &bn, &ks);
-  return (ks > 1 && !tc_clusterk()) ? (size_t)ks * L.B * L.Hout * L.Wout * L.Cout * sizeof(float) : 0;
+  return ks > 1 ? (size_t)ks * L.B * L.Hout * L.Wout * L.Cout * sizeof(float) : 0;
 }
 
 int tc_layer_prepare(ConvLayer& L, int num_sms) {
@@ -788,12 +454,10 @@ int tc_layer_prepare(ConvLayer& L, int num_sms) {
   if (make_weight_map(&L.tmB, L.w_tc, K, rows, L.block_n)) return -1;
   // output map for the TMA-store epilogue: deconv classes write every other pixel (element strides = conv strides)
   if (make_act_map(&L.tmO, L.out, L.Cout, L.Wout, L.Hout, L.B, L.tile_w, L.tile_h, L.transposed ? L.SW : 1, L.transposed ? L.SH : 1)) return -1;
-  L.tc2 = tc2_layer_config(L, num_sms, &L.tc2_groups, &L.tc2_ng);
-  if (L.tc2 && tc2_layer_prepare(L, g_encode)) return -1;
-  L.tc3 = !L.tc2 && tc3_layer_config(L, num_sms, &L.t3_tile_w, &L.t3_tile_h, &L.t3_mt, &L.t3_one);
+  L.tc3 = tc3_layer_config(L, num_sms, &L.t3_tile_w, &L.t3_tile_h, &L.t3_mt);
   if (L.tc3 && tc3_layer_prepare(L, g_encode)) return -1;
-  RYK_CHECK(L.ksplit == 1 || tc_layer_clusterk(L) || L.splitk_ws != nullptr, "split-K layer without a workspace");
-  if (L.ksplit > 1 && !tc_layer_clusterk(L)) {
+  RYK_CHECK(L.ksplit == 1 || L.splitk_ws != nullptr, "split-K layer without a workspace");
+  if (L.ksplit > 1) {
     if (make_ws_map(&L.tmW, L.splitk_ws, L.Cout, L.Wout, L.Hout, L.B, L.ksplit, L.tile_w, L.tile_h, L.transposed ? L.SW : 1, L.transposed ? L.SH : 1)) return -1;
   } else L.tmW = L.tmO;
   L.tc_ready = true;
@@ -809,28 +473,25 @@ static bool pdl_enabled() {
   if (v < 0) { const char* e = getenv("RYK_NO_PDL"); v = (e && atoi(e) != 0) ? 0 : 1; }
   return g_pdl_force >= 0 ? g_pdl_force != 0 : v != 0;
 }
-static int g_cluster_z = 1;                        // cluster dimension along grid z of the next launch_pdl (in-cluster split-K)
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int n = 0;
-  if (pdl_enabled()) { attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[n].val.programmaticStreamSerializationAllowed = 1; ++n; }
-  if (g_cluster_z > 1) { attr[n].id = cudaLaunchAttributeClusterDimension; attr[n].val.clusterDim.x = 1; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = (unsigned)g_cluster_z; ++n; }
-  cfg.attrs = attr; cfg.numAttrs = n;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
 int conv_tc_run(const ConvLayer& L, cudaStream_t st) {
   RYK_CHECK(L.tc_ready, "tc layer not prepared");
-  if (L.tc2) return conv_tc2_run(L, st, pdl_enabled());
   if (L.tc3) return conv_tc3_run(L, st, pdl_enabled());
   TcParams p;
-  p.transposed = L.transposed; p.B = L.B; p.Hout = L.Hout; p.Wout = L.Wout; p.Cout = L.Cout;
-  p.Hc = L.transposed ? L.Hin : L.Hout; p.Wc = L.transposed ? L.Win : L.Wout;
+  const int Hc = L.transposed ? L.Hin : L.Hout, Wc = L.transposed ? L.Win : L.Wout;    // class-local output grid
+  p.transposed = L.transposed; p.Cout = L.Cout;
   p.tile_w = L.tile_w; p.tile_h = L.tile_h;
-  p.tiles_w = (p.Wc + L.tile_w - 1) / L.tile_w; p.tiles_h = (p.Hc + L.tile_h - 1) / L.tile_h;
+  p.tiles_w = (Wc + L.tile_w - 1) / L.tile_w; p.tiles_h = (Hc + L.tile_h - 1) / L.tile_h;
   p.chunks0 = L.C0 / kBlockK; p.chunks1 = L.C1 / kBlockK;
   p.taps_w = L.transposed ? L.KW / L.SW : L.KW;
   p.ntaps = L.transposed ? (L.KH / L.SH) * (L.KW / L.SW) : L.KH * L.KW;
@@ -840,12 +501,8 @@ int conv_tc_run(const ConvLayer& L, cudaStream_t st) {
   p.ksplit = L.ksplit;
   int total_chunks = p.ntaps * (p.chunks0 + p.chunks1);
   p.chunks_per_split = (total_chunks + L.ksplit - 1) / L.ksplit;
-  p.act = L.act; p.scale = L.scale; p.shift = L.shift; p.out = (__half*)L.out;
-  const bool ck = tc_layer_clusterk(L);
-  p.ws = (L.ksplit > 1 && !ck) ? L.splitk_ws : nullptr;
-  p.cluster_k = ck ? 1 : 0;
-  g_cluster_z = ck ? L.ksplit : 1;
-  p.out_pixels = (size_t)L.B * L.Hout * L.Wout;
+  p.act = L.act; p.scale = L.scale; p.shift = L.shift;
+  p.ws = L.ksplit > 1 ? L.splitk_ws : nullptr;
 #ifdef RYK_DIAG
   { static int dbg = -1; if (dbg < 0) { const char* v = getenv("RYK_TC_DEBUG"); dbg = v ? atoi(v) : 0; } p.debug = dbg; }   // diagnostics builds only
 #else
@@ -853,34 +510,8 @@ int conv_tc_run(const ConvLayer& L, cudaStream_t st) {
 #endif
   size_t out_elems = (size_t)L.B * L.Hout * L.Wout * L.Cout;
   dim3 grid(L.B * p.tiles_w * p.tiles_h, L.Cout / L.block_n, classes * L.ksplit);
-  const int variant = tc_variant();
-  if (variant == 6) {
-    if (L.block_n == 128) RYK_CUDA(launch_pdl(k_conv_tc<128, 2, 3>, grid, dim3(kTcThreads), tc_smem_bytes<128, 2>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-    else RYK_CUDA(launch_pdl(k_conv_tc<64, 3, 3>, grid, dim3(kTcThreads), tc_smem_bytes<64, 3>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-  } else if (variant >= 3) {
-    int num_sms = 148;
-    cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, 0);
-    const int tiles_mn = L.B * p.tiles_w * p.tiles_h, n_tiles_n = L.Cout / L.block_n;
-    const int mt = variant == 5 ? 2 : 1;
-    const int total_tiles = ((tiles_mn + mt - 1) / mt) * n_tiles_n * classes * L.ksplit;
-    const int ctas = total_tiles < num_sms ? total_tiles : num_sms;
-    if (mt == 2) {
-      if (L.block_n == 256) k_conv_tc_persist<256, 2, 2><<<ctas, kTcThreads, tcp_smem_bytes<256, 2, 2>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-      else if (L.block_n == 128) k_conv_tc_persist<128, 4, 2><<<ctas, kTcThreads, tcp_smem_bytes<128, 4, 2>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-      else k_conv_tc_persist<64, 5, 2><<<ctas, kTcThreads, tcp_smem_bytes<64, 5, 2>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-    } else if (L.block_n == 256) k_conv_tc_persist<256, 3, 1><<<ctas, kTcThreads, tcp_smem_bytes<256, 3, 1>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-    else if (L.block_n == 128) k_conv_tc_persist<128, 6, 1><<<ctas, kTcThreads, tcp_smem_bytes<128, 6, 1>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-    else k_conv_tc_persist<64, 8, 1><<<ctas, kTcThreads, tcp_smem_bytes<64, 8, 1>(), st>>>(L.tmA0, L.tmA1, L.tmB, L.tmO, p, tiles_mn, n_tiles_n, total_tiles);
-  } else if (variant == 0) {
-    if (L.block_n == 256) RYK_CUDA(launch_pdl(k_conv_tc<256, 4, 1>, grid, dim3(kTcThreads), tc_smem_bytes<256, 4>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-    else if (L.block_n == 128) RYK_CUDA(launch_pdl(k_conv_tc<128, 6, 1>, grid, dim3(kTcThreads), tc_smem_bytes<128, 6>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-    else RYK_CUDA(launch_pdl(k_conv_tc<64, 6, 1>, grid, dim3(kTcThreads), tc_smem_bytes<64, 6>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-  } else {
-    if (L.block_n == 256) RYK_CUDA(launch_pdl(k_conv_tc<256, 2, 2>, grid, dim3(kTcThreads), tc_smem_bytes<256, 2>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-    else if (L.block_n == 128) RYK_CUDA(launch_pdl(k_conv_tc<128, 3, 2>, grid, dim3(kTcThreads), tc_smem_bytes<128, 3>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-    else RYK_CUDA(launch_pdl(k_conv_tc<64, 4, 2>, grid, dim3(kTcThreads), tc_smem_bytes<64, 4>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
-  }
-  g_cluster_z = 1;
+  if (L.block_n == 128) RYK_CUDA(launch_pdl(k_conv_tc<128, 3>, grid, dim3(kTcThreads), tc_smem_bytes<128, 3>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
+  else RYK_CUDA(launch_pdl(k_conv_tc<64, 4>, grid, dim3(kTcThreads), tc_smem_bytes<64, 4>(), st, L.tmA0, L.tmA1, L.tmB, L.tmO, L.tmW, p));
   RYK_CUDA(cudaGetLastError());
 #ifdef RYK_TC_TIMELINE
   cudaStreamCaptureStatus cap_ = cudaStreamCaptureStatusNone;

@@ -92,26 +92,23 @@ constexpr int kT3Threads = 352;    // warps 0-7 epilogue, 8 = scheduler + A load
 // One pipeline stage = one halo box (A) + the weight tiles of all taps that read it (B region, 32 KB) behind ONE full / empty
 // barrier pair: the MMA thread waits once per 8-16 MMAs.  (A first version with separate A / B rings waited per weight tile; its
 // timeline -- profiles/r02_halo_v1_timeline.txt -- showed the tensor pipe idling ~40 % of the time behind the issuing thread.)
-// ONE = one tile per CTA (grid = tiles, two CTAs per SM, no scheduler draws): at batch 1 a 384 x 512 layer has 1-3 tiles per SM, too few
-// to amortise a persistent CTA's un-overlapped prologue and last epilogue; two co-resident one-tile CTAs overlap them instead.  The
-// epilogue then stages its output in stage 0 (every load of the single tile has been consumed by the time the accumulator is ready).
-template <int MT, int STAGES, bool ONE = false> struct T3Smem {
+template <int MT, int STAGES> struct T3Smem {
   static constexpr uint32_t kASlot = (MT * 128 + 16) * 128;      // worst case tile_w = 16: (MT * 8 + 1) rows of 16 pixels
   static constexpr uint32_t kBRegion = 2 * 128 * 128;            // two 128-row (or four 64-row) weight tiles of 64 K
   static constexpr uint32_t kStage = kASlot + kBRegion;
-  static constexpr uint32_t kOut = ONE ? 0 : 128 * 128;          // one [128 pixels][64 channels] fp16 staging block
+  static constexpr uint32_t kOut = 128 * 128;                    // one [128 pixels][64 channels] fp16 staging block
   static constexpr uint32_t kBars = 2 * STAGES + 4 + 2 * kT3Sched;
   static constexpr size_t bytes = (size_t)STAGES * kStage + kOut + kBars * 8 + kT3Sched * 4 + 16 + 2 * 128 * 4 + 1024 + 64;
 };
 
-template <int MT, int STAGES, bool ONE>
-__global__ void __launch_bounds__(kT3Threads, ONE ? 2 : 1)
+template <int MT, int STAGES>
+__global__ void __launch_bounds__(kT3Threads, 1)
 k_conv_halo(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmB,
             const __grid_constant__ CUtensorMap tmO, const __grid_constant__ Tc3Params p) {
-  using S = T3Smem<MT, STAGES, ONE>;
+  using S = T3Smem<MT, STAGES>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint8_t* smem_out = ONE ? smem : smem + STAGES * S::kStage;
+  uint8_t* smem_out = smem + STAGES * S::kStage;
   uint64_t* full = (uint64_t*)(smem + STAGES * S::kStage + S::kOut);   // [STAGES] count 2: A loader + B loader (each arrive.expect_tx its bytes)
   uint64_t* empty = full + STAGES;                    // [STAGES] count 1: tcgen05.commit after the stage's MMAs
   uint64_t* t_full = empty + STAGES;                  // [2] accumulator stage ready for the epilogue
@@ -122,7 +119,7 @@ k_conv_halo(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CU
   uint32_t* tmem_ptr_smem = (uint32_t*)(s_tile + kT3Sched);
   float* s_scale = (float*)(((uintptr_t)(tmem_ptr_smem + 2) + 15) & ~(uintptr_t)15);     // [nblk * 64]
   float* s_shift = s_scale + 128;
-  constexpr uint32_t kTmemCols = ONE ? 128 : (MT == 2 ? 512 : 256);      // ONE: a single accumulator (two such CTAs + per-tap CTAs share an SM's 512 columns)
+  constexpr uint32_t kTmemCols = MT == 2 ? 512 : 256;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   pdl_trigger();
@@ -194,7 +191,7 @@ k_conv_halo(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CU
       }
       if (tile >= p.total_tiles) break;
       int draw = 0;
-      if (!ONE && lane == 0) draw = atomicAdd(p.tile_ctr, 1);    // in flight while this tile's loads are issued
+      if (lane == 0) draw = atomicAdd(p.tile_ctr, 1);    // in flight while this tile's loads are issued
       int v, n0, b, oy0, ox0;
       decode(tile, v, n0, b, oy0, ox0);
       const T3Program& P = p.prog[v];
@@ -212,7 +209,6 @@ k_conv_halo(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CU
           if (lane == 0) TL3(0, 10);
         }
       }
-      if (ONE) { tile = p.total_tiles; continue; }       // one tile per CTA: publish the end marker next
       draw = __shfl_sync(0xffffffffu, draw, 0);
       // total_tiles draws happen per launch (one per processed tile); the one that returns total_tiles - 1 is the last: re-arm
       if (lane == 0 && draw == p.total_tiles - 1) atomicExch(p.tile_ctr, 0);
@@ -392,12 +388,11 @@ k_conv_halo(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CU
 // ------------------------------------------------------------------------------------ host side
 static int t3_env(const char* name, int dflt) { const char* v = getenv(name); return v ? atoi(v) : dflt; }
 
-#define T3_LIST(X) X(1, 2, false) X(1, 3, false) X(1, 4, false) X(2, 2, false) X(2, 3, false) X(1, 2, true)
+constexpr int kT3Stages = 3;
 
 int tc3_init() {
-#define T3_ATTR(MT, ST, ON) RYK_CUDA(cudaFuncSetAttribute(k_conv_halo<MT, ST, ON>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3Smem<MT, ST, ON>::bytes));
-  T3_LIST(T3_ATTR)
-#undef T3_ATTR
+  RYK_CUDA(cudaFuncSetAttribute(k_conv_halo<1, kT3Stages>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3Smem<1, kT3Stages>::bytes));
+  RYK_CUDA(cudaFuncSetAttribute(k_conv_halo<2, kT3Stages>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3Smem<2, kT3Stages>::bytes));
   return 0;
 }
 
@@ -430,9 +425,10 @@ static T3Geom t3_geom(const ConvLayer& L, int tile_w, int mt, int num_sms) {
 // shape allows (unit tests).  Measured (profiles/r02_layer_bench_*.txt): the persistent kernel's main loop runs at ~107 clocks per
 // 128x128x16 MMA against ~170 for the per-tap kernel, but a CTA pays ~13k clocks of un-overlapped prologue + last epilogue; with fewer
 // than ~3 tiles per SM (batch 1, 384 x 512) the two-CTAs-per-SM per-tap kernel, which overlaps those phases, is faster.
-// RYK_TC3_MT / RYK_TC3_TW force the M tiles per CTA / the tile width (tuning).
-bool tc3_layer_config(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h, int* mt, bool* one) {
-  *one = false;
+// RYK_TC3_MT / RYK_TC3_TW force the M tiles per CTA / the tile width (unit tests).
+constexpr int kT3MinTilesPerSm = 3;
+
+bool tc3_layer_config(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h, int* mt) {
   const int mode = t3_env("RYK_TC3", 1);
   if (mode == 0) return false;
   const bool k2d = L.KH == 4 && L.KW == 4 && L.SH == 2 && L.SW == 2 && L.PH == 1 && L.PW == 1;
@@ -453,22 +449,7 @@ bool tc3_layer_config(const ConvLayer& L, int num_sms, int* tile_w, int* tile_h,
     }
   }
   if (best.tiles == 0) return false;
-  const int one_mode = t3_env("RYK_TC3_ONE", 0);      // 0 (default) = never: measured slower than the per-tap kernel on every batch-1 layer
-                                                       // (profiles/r02_layer_bench_one_tile.txt); 1 = where it has >= num_sms tiles, 2 = always (tests)
-  if (one_mode == 2 || (mode == 1 && best.tiles < t3_env("RYK_TC3_MIN_TILES_PER_SM", 3) * num_sms)) {
-    // too few tiles for persistent CTAs: one-tile CTAs (M = 128, two per SM) -- or the per-tap kernel
-    if (one_mode == 0) return false;
-    T3Geom g1; g1.tiles = 0; g1.cost = 1e30;
-    for (int tw = 8; tw <= 16; tw *= 2) {
-      if (Wc % tw != 0 || (force_tw && tw != force_tw) || Hc < (kBlockM / tw) / 2) continue;
-      T3Geom g = t3_geom(L, tw, 1, num_sms);
-      if (g.cost < g1.cost) g1 = g;
-    }
-    if (g1.tiles == 0) return false;
-    if (one_mode == 1 && g1.tiles < t3_env("RYK_TC3_ONE_MIN_TILES", num_sms)) return false;
-    *tile_w = g1.tile_w; *tile_h = g1.tile_h; *mt = 1; *one = true;
-    return true;
-  }
+  if (mode == 1 && best.tiles < kT3MinTilesPerSm * num_sms) return false;
   *tile_w = best.tile_w; *tile_h = best.tile_h; *mt = best.mt;
   return true;
 }
@@ -583,13 +564,13 @@ int conv_tc3_run(const ConvLayer& L, cudaStream_t st, bool pdl) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-  const int depth = t3_env("RYK_TC3_DEPTH", 1);        // 0 = two stages (smallest shared-memory footprint), 1 = default, 2 = deepest
-#define T3_LAUNCH(MTv, ST, ON) do { cfg.dynamicSmemBytes = T3Smem<MTv, ST, ON>::bytes; \
-    RYK_CUDA(cudaLaunchKernelEx(&cfg, k_conv_halo<MTv, ST, ON>, L.t3A0, L.t3A1, L.t3B, L.t3O, p)); } while (0)
-  if (L.t3_one) { cfg.gridDim = dim3(p.total_tiles); T3_LAUNCH(1, 2, true); }
-  else if (mt == 1) { if (depth == 0) T3_LAUNCH(1, 2, false); else if (depth == 1) T3_LAUNCH(1, 3, false); else T3_LAUNCH(1, 4, false); }
-  else { if (depth == 0) T3_LAUNCH(2, 2, false); else T3_LAUNCH(2, 3, false); }
-#undef T3_LAUNCH
+  if (mt == 1) {
+    cfg.dynamicSmemBytes = T3Smem<1, kT3Stages>::bytes;
+    RYK_CUDA(cudaLaunchKernelEx(&cfg, k_conv_halo<1, kT3Stages>, L.t3A0, L.t3A1, L.t3B, L.t3O, p));
+  } else {
+    cfg.dynamicSmemBytes = T3Smem<2, kT3Stages>::bytes;
+    RYK_CUDA(cudaLaunchKernelEx(&cfg, k_conv_halo<2, kT3Stages>, L.t3A0, L.t3A1, L.t3B, L.t3O, p));
+  }
   RYK_CUDA(cudaGetLastError());
 #ifdef RYK_TC_TIMELINE
   cudaStreamCaptureStatus cap_ = cudaStreamCaptureStatusNone;

@@ -1,5 +1,5 @@
 // tc_ptx.cuh -- inline-PTX wrappers shared by the tcgen05 convolution kernels (conv_tc.cu: one CTA per tile;
-// conv_tc2.cu: CTA pairs, cta_group::2): mbarriers, TMA loads, UMMA issue / commit, smem descriptors, PDL.
+// conv_tc3.cu: persistent halo kernel): mbarriers, TMA loads, UMMA issue / commit, smem descriptors, PDL.
 #pragma once
 #include <cuda.h>
 #include <stdint.h>
@@ -69,22 +69,8 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
       "}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
-// thread-block clusters: shared::cluster address of a CTA-local shared address in CTA `rank`, cluster rank, cluster-wide barrier
-__device__ __forceinline__ uint32_t cluster_map_rank(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
+// rank of this CTA in its thread-block cluster
 __device__ __forceinline__ uint32_t cluster_rank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_barrier() {
-  asm volatile("barrier.cluster.arrive.release;" ::: "memory");      // non-.aligned forms: callers may be divergent across warps
-  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
-}
-__device__ __forceinline__ float4 ld_cluster_f4(uint32_t addr) {
-  float4 v;
-  asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr) : "memory");
-  return v;
-}
 
 // K-major, 128B-swizzled operand: 8-row atoms of 1024 B (SBO), LBO unused, descriptor version 1 (sm_100)
 __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {

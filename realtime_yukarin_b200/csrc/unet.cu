@@ -179,7 +179,7 @@ int unet_forward(Engine* e, UNetPlan* p, cudaStream_t st, int first_layer, int l
     int rc = L.tc_ready ? conv_tc_run(L, st) : conv_direct_run(L, st);
     if (rc) return rc;
     if (prof && i == 14 && ev0) { RYK_CUDA(cudaEventRecord(ev1, st)); e->prof_events.emplace_back(ev0, ev1); }
-    e->launches += (L.tc_ready && L.ksplit > 1 && !tc_layer_clusterk(L)) ? 2 : 1;     // workspace split-K: kernel + reduce
+    e->launches += (L.tc_ready && L.ksplit > 1) ? 2 : 1;     // split-K: kernel + reduce
   }
   return 0;
 }

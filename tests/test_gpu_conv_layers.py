@@ -117,50 +117,6 @@ def test_stage1_last_layer_kernel(engine, case):
     assert err < 1e-4, err
 
 
-PAIR_CASES = [
-    # CTA-pair kernel (conv_tc2.cu, cta_group::2), forced with RYK_TC2=2: transposed, B, H, W, C0, C1, Cout, act
-    (0, 1, 32, 64, 64, 0, 128, 1),       # conv, N = 128, 4 pixel tiles (2 pairs)
-    (0, 2, 16, 16, 128, 0, 256, 1),      # conv, two N tiles, batch 2, 64-pixel images (tile covers two batch rows? no: 1 tile per image)
-    (0, 1, 48, 80, 64, 64, 128, 1),      # conv, two sources, ragged tile edges (24 x 40 outputs)
-    (1, 1, 12, 16, 128, 128, 64, 2),     # deconv, 4 fused parity classes of N = 64 (d6 shape family)
-    (1, 2, 24, 32, 64, 64, 128, 2),      # deconv, 2 fused classes of N = 128 (d5 shape family), batch 2
-    (1, 1, 3, 4, 256, 0, 256, 2),        # deconv, per-class N = 128 x 2 N tiles, ONE pixel tile -> padded pair
-    (1, 1, 20, 24, 64, 0, 64, 2),        # deconv, 4 classes, ragged edges, odd tile count
-    (1, 1, 48, 64, 256, 256, 256, 2),    # deconv, d4 shape family: 16 channel chunks per tap
-]
-
-
-@pytest.mark.parametrize('case', PAIR_CASES)
-def test_pair_kernel(engine, case):
-    """k_conv_tc2: UMMA M = 256 over a CTA pair, class-fused transposed convs; same tolerance as the one-CTA tcgen05 kernel."""
-    import os
-    tr, B, H, W, C0, C1, Cout, act = case
-    rng = np.random.default_rng(abs(hash(case)) % (2 ** 31))
-    in0 = rng.standard_normal((B, H, W, C0)).astype(np.float32)
-    in1 = rng.standard_normal((B, H, W, C1)).astype(np.float32) if C1 else None
-    Cin = C0 + C1
-    shape = (Cin, Cout, 4, 4) if tr else (Cout, Cin, 4, 4)
-    Wt = (rng.standard_normal(shape) / np.sqrt(Cin * 16 / (4 if tr else 1))).astype(np.float32)
-    scale = rng.uniform(0.8, 1.2, Cout).astype(np.float32)
-    shift = (0.1 * rng.standard_normal(Cout)).astype(np.float32)
-    ref = _ref(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act)
-    old = os.environ.get('RYK_TC2')
-    try:
-        os.environ['RYK_TC2'] = '0'
-        base, _ = engine.test_conv_layer(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act, use_tc=1)
-        os.environ['RYK_TC2'] = '2'
-        got, ms = engine.test_conv_layer(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act, use_tc=1, repeat=3)
-    finally:
-        if old is None:
-            os.environ.pop('RYK_TC2', None)
-        else:
-            os.environ['RYK_TC2'] = old
-    err, err_base = np.abs(got - ref).max(), np.abs(base - ref).max()
-    print('pair kernel', case, 'max err', err, '(one-CTA kernel', err_base, ') ms', ms)
-    assert err < 3e-2, err
-    assert np.abs(got - base).max() < 2e-2          # same fp16 operands, fp32 accumulation in a different order
-
-
 # The 14 k4 layers of the stage-2 U-Net exactly as the benchmarked forward runs them (base 64, Tp = 384 x 512 bins, batch 1):
 # same tile geometry, same split-K factor (ksplit is a function of the layer shape and the SM count only), same skip-concat
 # split of the decoder inputs.   name, transposed, H, W, C0, C1, Cout, act
@@ -191,7 +147,7 @@ def _ref32(in0, in1, W, scale, shift, transposed, act):
 
 @pytest.mark.parametrize('case', PRODUCTION_LAYERS, ids=[c[0] for c in PRODUCTION_LAYERS])
 def test_production_layer_shapes(engine, case):
-    """tcgen05 kernel (and, with RYK_TC_HALO default on, the halo kernel) on the shapes bench.py runs; inputs are fp16-representable
+    """tcgen05 kernel (and, where the default RYK_TC3=1 rule picks it, the halo kernel) on the shapes bench.py runs; inputs are fp16-representable
     so that the only differences from the float32 reference are accumulation order and the fp16 output rounding."""
     name, tr, H, W, C0, C1, Cout, act = case
     B = 2 if name.endswith('_b2_512') else 1
@@ -247,23 +203,17 @@ def test_halo_kernel(engine, case):
     scale = rng.uniform(0.8, 1.2, Cout).astype(np.float32)
     shift = (0.1 * rng.standard_normal(Cout)).astype(np.float32)
     ref = _ref(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act)
-    keys = ('RYK_TC3', 'RYK_TC3_MT', 'RYK_TC3_TW', 'RYK_TC3_DEPTH', 'RYK_TC3_ONE')
+    keys = ('RYK_TC3', 'RYK_TC3_MT', 'RYK_TC3_TW')
     old = {k: os.environ.get(k) for k in keys}
     try:
         os.environ['RYK_TC3'] = '0'
         base, _ = engine.test_conv_layer(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act, use_tc=1)
-        os.environ.update(RYK_TC3='2', RYK_TC3_MT=str(mt), RYK_TC3_TW=str(tw), RYK_TC3_ONE='0')
-        # depth 1 / 0: persistent CTAs with 3 / 2 stages; 'one': one tile per CTA, two CTAs per SM, staging aliased to stage 0
-        for depth in (1, 0, 'one'):
-            if depth == 'one':
-                os.environ.update(RYK_TC3='1', RYK_TC3_ONE='2')
-            else:
-                os.environ['RYK_TC3_DEPTH'] = str(depth)
-            got, ms = engine.test_conv_layer(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act, use_tc=1, repeat=3)
-            err, err_base = np.abs(got - ref).max(), np.abs(base - ref).max()
-            print('halo kernel', case, 'depth', depth, 'max err', err, '(per-tap kernel', err_base, ') ms', ms)
-            assert err < 3e-2, err
-            assert np.abs(got - base).max() < 2e-2
+        os.environ.update(RYK_TC3='2', RYK_TC3_MT=str(mt), RYK_TC3_TW=str(tw))
+        got, ms = engine.test_conv_layer(in0, in1, Wt, scale, shift, tr, 4, 2, 1, act, use_tc=1, repeat=3)
+        err, err_base = np.abs(got - ref).max(), np.abs(base - ref).max()
+        print('halo kernel', case, 'max err', err, '(per-tap kernel', err_base, ') ms', ms)
+        assert err < 3e-2, err
+        assert np.abs(got - base).max() < 2e-2
     finally:
         for k, v in old.items():
             if v is None:

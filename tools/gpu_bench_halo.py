@@ -1,4 +1,4 @@
-"""Layer-by-layer timing of the stage-2 k4 layers: per-tap kernel (RYK_TC3=0) vs the halo kernel in its ring-depth / tile variants.
+"""Layer-by-layer timing of the stage-2 k4 layers: per-tap kernel (RYK_TC3=0), the default choice, and the halo kernel with M = 128 / 256.
 Usage (GPU box): python tools/gpu_bench_halo.py [TP=384] ; prints one table, no correctness check (tests do that)."""
 import os, sys; sys.path.insert(0, '.')
 import numpy as np
@@ -16,11 +16,9 @@ for d in range(7):
     layers.append((f'd{d}', 1, Tp >> (7 - d), 512 >> (7 - d), c0, c1, base * dec[d]))
 only = os.environ.get('LAYERS')
 configs = [('per-tap', dict(RYK_TC3='0')), ('default', dict())]
-for tw in (8, 16):
-    configs.append((f'one-tile tw{tw}', dict(RYK_TC3='1', RYK_TC3_ONE='2', RYK_TC3_TW=str(tw))))
 for mt in (1, 2):
-    configs.append((f'persist mt{mt}', dict(RYK_TC3='2', RYK_TC3_ONE='0', RYK_TC3_DEPTH='1', RYK_TC3_MT=str(mt))))
-keys = ('RYK_TC3', 'RYK_TC3_MT', 'RYK_TC3_TW', 'RYK_TC3_DEPTH', 'RYK_TC3_ONE')
+    configs.append((f'persist mt{mt}', dict(RYK_TC3='2', RYK_TC3_MT=str(mt))))
+keys = ('RYK_TC3', 'RYK_TC3_MT', 'RYK_TC3_TW')
 print('layer      GFLOP ' + ' '.join(f'{n:>13s}' for n, _ in configs))
 tot = np.zeros(len(configs)); totf = 0.0
 for name, tr, H, W, C0, C1, Cout in layers:

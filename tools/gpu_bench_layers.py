@@ -25,7 +25,7 @@ for name, tr, H, W, C0, C1, Cout in layers:
     fl = 2.0 * 16 * Cin * Cout * (H * W if tr else Ho * Wo)
     tot += ms; totf += fl
     print(f'{name}: in {H}x{W}x{Cin} -> {Cout}: {ms * 1e3:7.1f} us  {fl / ms / 1e9:7.1f} TFLOP/s')
-print(f'TOTAL variant={os.environ.get("RYK_TC_VARIANT", "default")}: {tot * 1e3:.1f} us, {totf / tot / 1e9:.1f} TFLOP/s')
+print(f'TOTAL: {tot * 1e3:.1f} us, {totf / tot / 1e9:.1f} TFLOP/s')
 # edge layers (3x3): c0 = 1 -> 64 (fp32 in, fp16 out), out = 64 + 64 -> 1 (fp16 in, fp32 out)
 in0 = rng.standard_normal((1, Tp, 512, 1)).astype(np.float32)
 Wt = rng.standard_normal((64, 1, 3, 3)).astype(np.float32) / 3

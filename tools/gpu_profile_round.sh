@@ -7,5 +7,3 @@ if [ "$FULL" = "1" ]; then
   ncu --set full --clock-control none -s 720 -c 100 -f -o /tmp/${TAG}_full python bench.py --steps 4 --warmup 3 > gpurun_out/${TAG}_full_bench.log 2>&1
   python tools/ncu_summary.py /tmp/${TAG}_full.ncu-rep gpurun_out/${TAG}_ncu_full_one_step.csv
 fi
-RYK_TC2=1 ncu --set full --clock-control none -k regex:k_conv_tc2 -c 5 -f -o /tmp/${TAG}_pair python tools/gpu_bench_layers.py > gpurun_out/${TAG}_pair_layers.log 2>&1
-python tools/ncu_summary.py /tmp/${TAG}_pair.ncu-rep gpurun_out/${TAG}_ncu_full_pair_kernel.csv
