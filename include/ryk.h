@@ -242,6 +242,10 @@ int ryk_debug_synth_timebase(ryk_engine* e, int synth_id, int n, double* if0, do
  * of the most recent analysis that used the (n, fs, frame_period, f0_floor, f0_ceil) plan. */
 int ryk_debug_dio(ryk_engine* e, int n, int fs, double frame_period_ms, double f0_floor, double f0_ceil,
                   double* f0_raw, double* cand, double* score, int* counts);
+/* StoneMask alone on caller-given f0 estimates (frames values, frame i at i * frame_period_ms), shared memory sized from f0_floor
+ * as in analysis: an estimate below f0_floor whose FFT would not fit is returned unrefined. */
+int ryk_debug_stonemask(ryk_engine* e, const float* wave_host, int n, int fs, double frame_period_ms, double f0_floor,
+                        const double* f0_in, int frames, double* f0_out);
 /* Harvest internals of the most recent analysis with this plan (engine in f0 method 1): info = {channels, 1 ms frames, decimated
  * length, fft size, candidate columns, decimation ratio, used columns}; y [info[2]], raw [channels][frames], cand / score
  * [frames][columns] (after refinement and removal), best / basic [frames], f0_raw [n / hop + 1] (before StoneMask).  Any may be NULL. */

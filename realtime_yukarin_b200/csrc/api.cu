@@ -755,6 +755,27 @@ int ryk_debug_dio(ryk_engine* h, int n, int fs, double fp, double f0_floor, doub
   return dio_plan_debug_copy(plan, f0_raw, cand, score, counts, e->stream);
 }
 
+int ryk_debug_stonemask(ryk_engine* h, const float* wave, int n, int fs, double fp, double f0_floor, const double* f0_in, int frames,
+                        double* f0_out) {
+  Engine* e = E(h);
+  RYK_CUDA(cudaSetDevice(e->device));
+  RYK_CHECK(n > 0 && frames > 0, "empty input");
+  void* scratch = nullptr;
+  size_t need = arena_need({sizeof(float) * n, sizeof(double) * frames, sizeof(double) * frames});
+  if (engine_scratch(e, need, &scratch)) return -1;
+  Arena A(scratch);
+  float* d_x = A.take<float>(n);
+  double* d_in = A.take<double>(frames);
+  double* d_out = A.take<double>(frames);
+  RYK_CUDA(cudaMemcpyAsync(d_x, wave, sizeof(float) * n, cudaMemcpyHostToDevice, e->stream));
+  RYK_CUDA(cudaMemcpyAsync(d_in, f0_in, sizeof(double) * frames, cudaMemcpyHostToDevice, e->stream));
+  if (stonemask_run(e, d_x, n, fs, fp, f0_floor, d_in, d_out, frames, e->stream)) return -1;
+  e->launches += 1;
+  RYK_CUDA(cudaMemcpyAsync(f0_out, d_out, sizeof(double) * frames, cudaMemcpyDeviceToHost, e->stream));
+  RYK_CUDA(cudaStreamSynchronize(e->stream));
+  return 0;
+}
+
 // ---- diagnostics: one conv / transposed-conv layer in isolation (unit parity + profiling) -------
 // in0/in1: host fp32 NHWC [B][Hin][Win][C0|C1]; W: Chainer layout; out: host fp32 NHWC [B][Hout][Wout][Cout].
 // use_tc = 1 runs the FP16 tcgen05 kernel (activations rounded to fp16), 0 the FP32 CUDA-core kernel.

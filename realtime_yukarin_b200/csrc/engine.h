@@ -67,6 +67,8 @@ int dio_plan_create(Engine* e, int n, int fs, double frame_period, double f0_flo
 void dio_plan_free(DioPlan* p);
 int dio_get_plan(Engine* e, int n, int fs, double frame_period, double f0_floor, double f0_ceil, DioPlan** out);
 int dio_stonemask_run(Engine* e, DioPlan* p, const float* d_x, cudaStream_t st);
+int stonemask_run(Engine* e, const float* d_x, int n, int fs, double frame_period, double f0_floor, const double* d_f0_in,
+                  double* d_f0_out, int frames, cudaStream_t st);
 const double* dio_plan_f0(DioPlan* p);      // refined f0 (double) after dio_stonemask_run
 double* dio_plan_f0_mut(DioPlan* p);
 int dio_plan_frames(DioPlan* p);

@@ -195,25 +195,35 @@ __device__ inline double stonemask_fix(const double* power, const double* numer,
   return num / (den + kSafeMin);
 }
 
-// one CTA per frame; smem: 2 * 4096 double2 (main / diff spectra) + 2 * 2049 doubles
+// StoneMask's FFT size for an f0 estimate of f0i (> 0)
+__host__ __device__ inline int stonemask_fft_size(int fs, double f0i) {
+  int half = (int)(1.5 * fs / f0i + 1.0);
+  // NB: device pow() is not exact for integer powers (2 ulp): a truncated 2047 would wreck the FFT. Shift instead.
+  return 1 << (2 + (int)(log(half * 2.0 + 1.0) / kLog2));
+}
+
+// one CTA per frame; smem: 2 * fft_cap double2 (main / diff spectra) + 64 bytes, which keeps stonemask_fix's reads of bins up to
+// fft_size (a harmonic of the tentative f0 above Nyquist) inside the allocation, as the former separate arrays did.  fft_cap is the FFT size of the plan's lowest f0 (2048 at
+// 24 kHz / 71 Hz); a frame whose f0 would need a larger transform keeps its unrefined estimate.
 __global__ void __launch_bounds__(256) k_stonemask(const float* __restrict__ x, int x_length, int fs, double frame_period,
                                                   const double* __restrict__ f0_in, double* __restrict__ f0_out,
-                                                  const double2* __restrict__ tw) {
+                                                  const double2* __restrict__ tw, int fft_cap) {
   extern __shared__ double2 sm2[];
   int frame = blockIdx.x;
   double f0i = f0_in[frame];
   if (f0i <= 40.0 || f0i > fs / 12.0) { if (threadIdx.x == 0) f0_out[frame] = 0.0; return; }
+  int fft_size = stonemask_fft_size(fs, f0i);
+  if (fft_size > fft_cap) { if (threadIdx.x == 0) f0_out[frame] = f0i; return; }
   double pos = frame * frame_period / 1000.0;
   int half = (int)(1.5 * fs / f0i + 1.0);
   double wlen_time = (2.0 * half + 1.0) / fs;
   int blen = half * 2 + 1;
-  // NB: device pow() is not exact for integer powers (2 ulp): a truncated 2047 would wreck the FFT. Shift instead.
-  int fft_size = 1 << (2 + (int)(log(half * 2.0 + 1.0) / kLog2));
   int lg = ilog2(fft_size);
   double2* A = sm2;                 // main
-  double2* B = sm2 + 4096;          // diff
-  double* power = (double*)(sm2 + 8192);
-  double* numer = power + 2049;
+  double2* B = sm2 + fft_cap;       // diff
+  // only bins 0..fft/2 of each spectrum are read: power and numer go to the upper halves (fft/2 - 1 double2 >= fft/2 + 1 doubles)
+  double* power = (double*)(A + fft_size / 2 + 1);
+  double* numer = (double*)(B + fft_size / 2 + 1);
   int basic_index = matlab_round((pos + (double)(-half) / fs) * fs + 0.001);
   auto mainw = [&](int i) {
     double tmp = ((basic_index + i) - 1.0) / fs - pos;
@@ -385,6 +395,26 @@ __global__ void __launch_bounds__(256) k_cheaptrick(const float* __restrict__ x,
 }
 
 // ------------------------------------------------------------------------------------ D4C
+// block_sum of two values at once: the same warp trees and the same fixed-order pass over the warp totals as two block_sum() calls
+// (bit-identical results), at the barriers of one.
+__device__ inline double2 d4c_block_sum2(double a, double b, double* scratch) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
+  a = warp_sum(a);
+  b = warp_sum(b);
+  __syncthreads();
+  if (lane == 0) { scratch[w] = a; scratch[32 + w] = b; }
+  __syncthreads();
+  if (w == 0) {
+    double ra = warp_sum(lane < nw ? scratch[lane] : 0.0);
+    double rb = warp_sum(lane < nw ? scratch[32 + lane] : 0.0);
+    if (lane == 0) { scratch[0] = ra; scratch[1] = rb; }
+  }
+  __syncthreads();
+  const double2 r = make_double2(scratch[0], scratch[1]);
+  __syncthreads();
+  return r;
+}
+
 // windowed waveform into A[i].x (i < fft), zero elsewhere; returns after DC-weight removal.
 __device__ inline void d4c_window_smem(double2* A, int fft_size, const float* __restrict__ x, int x_length, int fs,
                                        double cf0, double pos, bool blackman, double ratio, double* scratch) {
@@ -403,9 +433,8 @@ __device__ inline void d4c_window_smem(double2* A, int fft_size, const float* __
     }
     A[i] = make_double2(v, wv);
   }
-  double s1 = block_sum(w1, scratch);
-  double s2 = block_sum(w2, scratch);
-  double coef = s1 / s2;
+  const double2 s12 = d4c_block_sum2(w1, w2, scratch);
+  double coef = s12.x / s12.y;
   for (int i = threadIdx.x; i < fft_size; i += blockDim.x) {
     double2 v = A[i];
     A[i] = make_double2(i <= half * 2 ? v.x - v.y * coef : 0.0, 0.0);
@@ -449,49 +478,100 @@ __device__ inline void d4c_centroid_smem(double2* A, int fft_size, int lg, const
   __syncthreads();
 }
 
-// bitonic sort (ascending) of v[0..n2) in smem, n2 power of two.  Warp w owns the contiguous segment [seg w, seg (w + 1)): every
-// compare-exchange with distance j < seg stays inside one warp's segment and needs only __syncwarp(); block barriers remain for the
-// log2(n2 / seg) widest distances of each merge (n2 = 2048, 16 warps: 15 block barriers instead of 67; same network, same result).
-__device__ inline void bitonic_sort_smem(double* v, int n2) {
-  const int nw = blockDim.x >> 5, w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  const int seg = n2 / nw;
-  if (seg < 32 || seg * nw != n2) {           // small arrays: the plain one-barrier-per-stage form
-    for (int k = 2; k <= n2; k <<= 1) {
-      for (int j = k >> 1; j > 0; j >>= 1) {
-        __syncthreads();
-        for (int i = threadIdx.x; i < n2; i += blockDim.x) {
-          int ixj = i ^ j;
-          if (ixj > i) {
-            double a = v[i], b = v[ixj];
-            bool up = (i & k) == 0;
-            if ((a > b) == up) { v[i] = b; v[ixj] = a; }
-          }
+// Coarse aperiodicity needs, per band, the sum of the m smallest of its n band powers and the sum of all n.  No sort: an 8-bit radix
+// select over the IEEE-754 bit patterns (non-negative doubles order like their uint64 patterns) finds the m-th smallest value t of
+// each band, and then sum_m = sum(v < t) + (m - #{v < t}) * t, which counts ties with t exactly.  The nb <= kD4cMaxBands bands are
+// selected together, one block barrier per digit for all of them; every warp scans the histograms itself, so no second barrier.
+// hist: 3 * nb * 256 ints (a histogram is zeroed two digits after it was read).  red: >= 16 * (blockDim.x / 32) doubles.
+// Sums are taken in a fixed order (per-thread index order, warp trees, warps in order): the result does not depend on timing.
+constexpr int kD4cMaxBands = 5;     // fmin(15000, fs/2 - 3000) / 3000
+__device__ inline void d4c_select_sums(double* const* p, int nb, int n, int m, int* hist, double* red, double* sum_m, double* sum_all) {
+  const int T = blockDim.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = T >> 5;
+  unsigned long long prefix[kD4cMaxBands];
+  int rank[kD4cMaxBands];                 // rank of the wanted value among the values that still match prefix
+#pragma unroll
+  for (int b = 0; b < kD4cMaxBands; ++b) { prefix[b] = 0ull; rank[b] = m - 1; }
+  for (int i = threadIdx.x; i < nb * 256; i += T) hist[i] = 0;
+  __syncthreads();
+  for (int pass = 0; pass < 8; ++pass) {
+    const int shift = 56 - 8 * pass;
+    int* H = hist + (pass % 3) * nb * 256;
+    int* Hn = hist + ((pass + 1) % 3) * nb * 256;
+    for (int i = threadIdx.x; i < nb * 256; i += T) Hn[i] = 0;
+#pragma unroll
+    for (int b = 0; b < kD4cMaxBands; ++b) {
+      if (b >= nb) break;
+      for (int i0 = 0; i0 < n; i0 += T) {          // warp-uniform trip count: __match_any_sync needs the whole warp
+        const int i = i0 + threadIdx.x;
+        int bin = -1;
+        if (i < n) {
+          const unsigned long long key = (unsigned long long)__double_as_longlong(p[b][i]);
+          if (pass == 0 || (key >> (shift + 8)) == (prefix[b] >> (shift + 8))) bin = (int)((key >> shift) & 255ull);
         }
+        const unsigned same = __match_any_sync(0xffffffffu, bin);
+        if (bin >= 0 && lane == __ffs(same) - 1) atomicAdd(&H[b * 256 + bin], __popc(same));
       }
     }
     __syncthreads();
-    return;
+#pragma unroll
+    for (int b = 0; b < kD4cMaxBands; ++b) {
+      if (b >= nb) break;
+      const int4 c0 = *(const int4*)&H[b * 256 + lane * 8];
+      const int4 c1 = *(const int4*)&H[b * 256 + lane * 8 + 4];
+      const int c[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
+      const int tot = c[0] + c[1] + c[2] + c[3] + c[4] + c[5] + c[6] + c[7];
+      int incl = tot;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
+      const int L = __ffs(__ballot_sync(0xffffffffu, incl > rank[b])) - 1;   // the lane whose 8 bins hold the wanted rank
+      int digit = 0, below = incl - tot;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        if (rank[b] < below + c[j]) { digit = lane * 8 + j; break; }
+        below += c[j];
+      }
+      digit = __shfl_sync(0xffffffffu, digit, L);
+      below = __shfl_sync(0xffffffffu, below, L);
+      prefix[b] |= (unsigned long long)digit << shift;
+      rank[b] -= below;
+    }
+  }
+  // prefix[b] is now the bit pattern of the m-th smallest value of band b
+#pragma unroll
+  for (int b = 0; b < kD4cMaxBands; ++b) {
+    if (b >= nb) break;
+    double s_lt = 0.0, s_all = 0.0, c_lt = 0.0;
+    for (int i = threadIdx.x; i < n; i += T) {
+      const double v = p[b][i];
+      s_all += v;
+      if ((unsigned long long)__double_as_longlong(v) < prefix[b]) { s_lt += v; c_lt += 1.0; }
+    }
+    s_lt = warp_sum(s_lt); s_all = warp_sum(s_all); c_lt = warp_sum(c_lt);
+    if (lane == 0) { red[w * 16 + 3 * b] = s_lt; red[w * 16 + 3 * b + 1] = s_all; red[w * 16 + 3 * b + 2] = c_lt; }
   }
   __syncthreads();
-  bool prev_block = false;
-  for (int k = 2; k <= n2; k <<= 1) {
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      const bool block_stage = j >= seg;
-      if (block_stage || prev_block) __syncthreads(); else __syncwarp();
-      prev_block = block_stage;
-      for (int m = 0; m < seg; m += 32) {
-        const int i = seg * w + m + l;
-        const int ixj = i ^ j;
-        if (ixj > i) {
-          double a = v[i], b = v[ixj];
-          bool up = (i & k) == 0;
-          if ((a > b) == up) { v[i] = b; v[ixj] = a; }
-        }
-      }
+#pragma unroll
+  for (int b = 0; b < kD4cMaxBands; ++b) {
+    if (b < nb && threadIdx.x == 32 * b) {          // one thread per band, each in its own warp
+      double s_lt = 0.0, s_all = 0.0, c_lt = 0.0;
+      for (int k = 0; k < nw; ++k) { s_lt += red[k * 16 + 3 * b]; s_all += red[k * 16 + 3 * b + 1]; c_lt += red[k * 16 + 3 * b + 2]; }
+      sum_m[b] = s_lt + (m - c_lt) * __longlong_as_double((long long)prefix[b]);
+      sum_all[b] = s_all;
     }
   }
   __syncthreads();
 }
+
+#ifdef RYK_D4C_TIMELINE
+// diagnostics build only (RYK_NVCC_EXTRA=-DRYK_D4C_TIMELINE): %globaltimer stamps of k_d4c's phases, thread 0 of each CTA,
+// dumped to RYK_D4C_TIMELINE_FILE after each launch outside a graph capture.  A frame that stops early leaves its later slots 0.
+constexpr int kD4cTlMaxCtas = 1024, kD4cTlSlots = 16;
+__device__ unsigned long long g_d4c_tl[kD4cTlMaxCtas * kD4cTlSlots];
+#define D4C_TL(slot) do { if (threadIdx.x == 0 && blockIdx.x < kD4cTlMaxCtas) { unsigned long long t_; \
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); g_d4c_tl[blockIdx.x * kD4cTlSlots + (slot)] = t_; } } while (0)
+#else
+#define D4C_TL(slot) do {} while (0)
+#endif
 
 // one CTA (512 threads) per frame
 __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_length, int fs, double frame_period,
@@ -514,11 +594,15 @@ __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_
   double* t1 = gd + alen;             // temp
   double* t2 = t1 + alen;             // temp
   double* seg = t2 + alen;            // smoothing scratch (hb + 2*boundary + 1)
-  double* scratch = seg + d4c_seg_len(fft_d4c, fs);   // blockDim.x + 32
+  double* nwin = seg + d4c_seg_len(fft_d4c, fs);      // Nuttall band window (window_length <= hb values)
+  double* coarse = nwin + alen;       // coarse aperiodicity (nap + 2) and the per-band sums (2 kD4cMaxBands)
+  double* scratch = coarse + 24;      // blockDim.x + 32
+  int* hist = (int*)(((uintptr_t)(scratch + 512 + 64) + 15) & ~(uintptr_t)15);   // radix-select histograms, 3 * nap * 256 (int4 reads)
   double f0v = f0[frame];
   double pos = frame * frame_period / 1000.0;
   const float unvoiced = (float)(1.0 - kSafeMin);
   bool skip = f0v == 0.0;
+  D4C_TL(0);
   if (!skip) {
     // D4C LoveTrain
     int lg = ilog2(lt_fft);
@@ -533,10 +617,11 @@ __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_
       p2 += pw;
       if (i <= b1) p1 += pw;
     }
-    double s1 = block_sum(p1, scratch), s2 = block_sum(p2, scratch);
-    double ap0 = s1 / s2;
+    const double2 s12 = d4c_block_sum2(p1, p2, scratch);
+    double ap0 = s12.x / s12.y;
     skip = ap0 <= threshold;     // NaN compares false, exactly like the CPU code path
   }
+  D4C_TL(1);
   if (skip) {
     for (int i = threadIdx.x; i < nb_out; i += blockDim.x) out[i] = unvoiced;
     return;
@@ -544,9 +629,11 @@ __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_
   int lg = ilog2(fft_d4c);
   double cf0 = f0v > 47.0 ? f0v : 47.0;
   d4c_centroid_smem(A, fft_d4c, lg, x, x_length, fs, cf0, pos - 0.25 / cf0, t1, t2, sc, false, scratch, tw);
+  D4C_TL(2);
   d4c_centroid_smem(A, fft_d4c, lg, x, x_length, fs, cf0, pos + 0.25 / cf0, t1, t2, sc, true, scratch, tw);
   if (threadIdx.x == 0) sc[hb] = 0.0;
   dc_correction_smem(sc, cf0, fs, fft_d4c);
+  D4C_TL(3);
   // smoothed power spectrum
   d4c_window_smem(A, fft_d4c, x, x_length, fs, cf0, pos, false, 4.0, scratch);
   fft_smem(A, fft_d4c, lg, -1, tw);
@@ -554,49 +641,68 @@ __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_
   if (threadIdx.x == 0) sps[hb] = 0.0;
   dc_correction_smem(sps, cf0, fs, fft_d4c);
   linear_smoothing_smem(sps, sps, cf0, fs, fft_d4c, seg, scratch);
+  D4C_TL(4);
   // static group delay
   for (int i = threadIdx.x; i < hb; i += blockDim.x) gd[i] = sc[i] / sps[i];
   linear_smoothing_smem(gd, gd, cf0 / 2.0, fs, fft_d4c, seg, scratch);
   linear_smoothing_smem(gd, t1, cf0, fs, fft_d4c, seg, scratch);
   for (int i = threadIdx.x; i < hb; i += blockDim.x) gd[i] -= t1[i];
   __syncthreads();
-  // coarse aperiodicity
+  D4C_TL(5);
+  // coarse aperiodicity: per band, the power spectrum of a Nuttall-windowed slice of gd; two bands share one complex FFT
+  // (band b in the real part, band b + 1 in the imaginary part, split by Hermitian symmetry as in d4c_centroid_smem)
   const int nap = (int)(fmin(15000.0, fs / 2.0 - 3000.0) / 3000.0);
   const int window_length = (int)(3000.0 * fft_d4c / fs) * 2 + 1;
   const int half_wl = window_length / 2;
   const int boundary = matlab_round(fft_d4c * 8.0 / window_length);
-  double* coarse = t2;                // nap + 2 values
-  double* srt = (double*)A;           // 2*maxfft doubles available; sort buffer of 2048
-  if (threadIdx.x == 0) { coarse[0] = -60.0; coarse[nap + 1] = -kSafeMin; }
-  for (int b = 0; b < nap; ++b) {
-    int center = (int)(3000.0 * (b + 1) * fft_d4c / fs);
+  for (int i = threadIdx.x; i < window_length; i += blockDim.x) {
+    double tmp = i / (window_length - 1.0);
+    nwin[i] = 0.355768 - 0.487396 * cos(2.0 * kPi * tmp) + 0.144232 * cos(4.0 * kPi * tmp) - 0.012604 * cos(6.0 * kPi * tmp);
+  }
+  double* const bp[kD4cMaxBands] = {sc, sps, t1, t2, seg};   // band power spectra (hb values each); sc / sps / t1 / t2 / seg are free now
+  for (int b = 0; b < nap; b += 2) {
+    const bool pair = b + 1 < nap;
+    const int c0 = (int)(3000.0 * (b + 1) * fft_d4c / fs) - half_wl;
+    const int c1 = (int)(3000.0 * (b + 2) * fft_d4c / fs) - half_wl;
     __syncthreads();
     for (int i = threadIdx.x; i < fft_d4c; i += blockDim.x) {
-      double v = 0.0;
-      if (i <= half_wl * 2) {
-        double tmp = i / (window_length - 1.0);
-        double w = 0.355768 - 0.487396 * cos(2.0 * kPi * tmp) + 0.144232 * cos(4.0 * kPi * tmp) - 0.012604 * cos(6.0 * kPi * tmp);
-        v = gd[center - half_wl + i] * w;
+      double v0 = 0.0, v1 = 0.0;
+      if (i < window_length) {
+        v0 = gd[c0 + i] * nwin[i];
+        if (pair) v1 = gd[c1 + i] * nwin[i];
       }
-      A[i] = make_double2(v, 0.0);
+      A[i] = make_double2(v0, v1);
     }
     fft_smem(A, fft_d4c, lg, -1, tw);
-    // power spectrum -> t1 (hb values), then sort in srt (padded to pow2 with +inf)
-    for (int i = threadIdx.x; i < hb; i += blockDim.x) { double2 v = A[i]; t1[i] = v.x * v.x + v.y * v.y; }
-    __syncthreads();
-    int n2 = 1; while (n2 < hb) n2 <<= 1;
-    for (int i = threadIdx.x; i < n2; i += blockDim.x) srt[i] = i < hb ? t1[i] : INFINITY;
-    bitonic_sort_smem(srt, n2);
-    // cumulative sums at two indices
-    int idx_a = fft_d4c / 2 - boundary - 1, idx_b = fft_d4c / 2;
-    double pa = 0.0, pb = 0.0;
-    for (int i = threadIdx.x; i <= idx_b; i += blockDim.x) { double v = srt[i]; pb += v; if (i <= idx_a) pa += v; }
-    double sa = block_sum(pa, scratch), sb = block_sum(pb, scratch);
-    if (threadIdx.x == 0) {
-      double ca = 10 * log10(sa / sb);
-      coarse[1 + b] = fmin(0.0, ca + (cf0 - 100) / 50.0);
+    D4C_TL(6 + b / 2);
+    double* p0 = b == 0 ? sc : b == 2 ? t1 : seg;
+    double* p1 = b == 0 ? sps : t2;
+    for (int k = threadIdx.x; k < hb; k += blockDim.x) {
+      const double2 z = A[k];
+      if (pair) {
+        const double2 zc = A[(fft_d4c - k) & (fft_d4c - 1)];
+        const double xr = 0.5 * (z.x + zc.x), xi = 0.5 * (z.y - zc.y);
+        const double yr = 0.5 * (z.y + zc.y), yi = -0.5 * (z.x - zc.x);
+        p0[k] = xr * xr + xi * xi;
+        p1[k] = yr * yr + yi * yi;
+      } else {
+        p0[k] = z.x * z.x + z.y * z.y;
+      }
     }
   }
+  __syncthreads();
+  D4C_TL(9);
+  // pa: the fft/2 - boundary smallest of the hb band powers, pb: all of them (the CPU code sorts and takes two cumulative sums)
+  double* sum_m = coarse + kD4cMaxBands + 2;
+  double* sum_all = sum_m + kD4cMaxBands;
+  d4c_select_sums(bp, nap, hb, fft_d4c / 2 - boundary, hist, scratch, sum_m, sum_all);
+  D4C_TL(10);
+  if (threadIdx.x == 0) {
+    coarse[0] = -60.0;
+    coarse[nap + 1] = -kSafeMin;
+    for (int b = 0; b < nap; ++b) coarse[1 + b] = fmin(0.0, 10 * log10(sum_m[b] / sum_all[b]) + (cf0 - 100) / 50.0);
+  }
+  D4C_TL(11);
   __syncthreads();
   for (int i = threadIdx.x; i < nb_out; i += blockDim.x) {
     double fx = (double)i * fs / fft_size_out;
@@ -615,6 +721,7 @@ __global__ void __launch_bounds__(512) k_d4c(const float* __restrict__ x, int x_
     double v = coarse[k - 1] + s * (coarse[k] - coarse[k - 1]);
     out[i] = (float)pow(10.0, v / 20.0);
   }
+  D4C_TL(15);
 }
 
 // f0 / voiced outputs (float32 / uint8), trimmed to n_out frames
@@ -699,14 +806,22 @@ int dio_plan_create(Engine* e, int n, int fs, double frame_period, double f0_flo
   return 0;
 }
 
+// StoneMask refinement of `frames` f0 estimates.  Shared memory is sized for the largest FFT an f0 >= f0_floor can need (DIO and
+// Harvest return no nonzero f0 below f0_floor), capped at the twiddle table's size.
+int stonemask_run(Engine* e, const float* d_x, int n, int fs, double frame_period, double f0_floor, const double* d_f0_in,
+                  double* d_f0_out, int frames, cudaStream_t st) {
+  int fft_cap = stonemask_fft_size(fs, fmax(f0_floor, 40.0));
+  if (fft_cap > kTwiddleN) fft_cap = kTwiddleN;
+  k_stonemask<<<frames, 256, sizeof(double2) * 2 * fft_cap + 64, st>>>(d_x, n, fs, frame_period, d_f0_in, d_f0_out, e->d_twiddle, fft_cap);
+  RYK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 // DIO + StoneMask: x (device float32, n samples) -> plan->d_f0r (double, f0_length frames). Stream-ordered, no sync.
 int dio_stonemask_run(Engine* e, DioPlan* p, const float* d_x, cudaStream_t st) {
-  const size_t sm_smem = sizeof(double2) * 8192 + sizeof(double) * 2 * 2049 + 64;
   if (p->harvest) {                                  // Harvest replaces DIO as the contour StoneMask refines
     if (harvest_run(e, p->harvest, d_x, p->d_f0, st)) return -1;
-    k_stonemask<<<p->f0_length, 256, sm_smem, st>>>(d_x, p->n, p->fs, p->frame_period, p->d_f0, p->d_f0r, e->d_twiddle);
-    RYK_CUDA(cudaGetLastError());
-    return 0;
+    return stonemask_run(e, d_x, p->n, p->fs, p->frame_period, p->f0_floor, p->d_f0, p->d_f0r, p->f0_length, st);
   }
   int nbins = p->fft_size / 2 + 1;
   if (cufft_ok(cufftSetStream(p->fwd, st), "set stream")) return -1;
@@ -723,10 +838,7 @@ int dio_stonemask_run(Engine* e, DioPlan* p, const float* d_x, cudaStream_t st) 
       p->d_boundary, p->d_cand, p->d_score);
   k_dio_fix<<<1, 256, 0, st>>>(p->d_cand, p->d_score, p->nbands, p->f0_length, p->frame_period, p->f0_floor, p->d_scratch,
                                p->d_iscratch, p->d_f0);
-  size_t smem = sizeof(double2) * 8192 + sizeof(double) * 2 * 2049 + 64;
-  k_stonemask<<<p->f0_length, 256, smem, st>>>(d_x, p->n, p->fs, p->frame_period, p->d_f0, p->d_f0r, e->d_twiddle);
-  RYK_CUDA(cudaGetLastError());
-  return 0;
+  return stonemask_run(e, d_x, p->n, p->fs, p->frame_period, p->f0_floor, p->d_f0, p->d_f0r, p->f0_length, st);
 }
 
 const double* dio_plan_f0(DioPlan* p) { return p->d_f0r; }
@@ -753,11 +865,13 @@ size_t d4c_smem_bytes(int fs) {
   int lt_fft = (int)pow(2.0, 1.0 + (int)(log(3.0 * fs / 40.0 + 1) / kLog2));
   int maxfft = fft_d4c > lt_fft ? fft_d4c : lt_fft;
   int hb = fft_d4c / 2 + 1;
-  return sizeof(double2) * maxfft + sizeof(double) * (5 * (hb + 8) + d4c_seg_len(fft_d4c, fs) + 512 + 64);
+  int nap = (int)(fmin(15000.0, fs / 2.0 - 3000.0) / 3000.0);
+  return sizeof(double2) * maxfft + sizeof(double) * (6 * (hb + 8) + d4c_seg_len(fft_d4c, fs) + 24 + 512 + 64) +
+         16 + sizeof(int) * 3 * nap * 256;
 }
 
 int analysis_kernels_init() {
-  RYK_CUDA(cudaFuncSetAttribute(k_stonemask, cudaFuncAttributeMaxDynamicSharedMemorySize, 170 * 1024));
+  RYK_CUDA(cudaFuncSetAttribute(k_stonemask, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * kTwiddleN * (int)sizeof(double2) + 64));
   RYK_CUDA(cudaFuncSetAttribute(k_cheaptrick, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
   RYK_CUDA(cudaFuncSetAttribute(k_d4c, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   return 0;
@@ -774,7 +888,24 @@ int spectral_analysis_run(Engine* e, const float* d_x, int n, int fs, double fra
                                                                       n_out, d_sp, d_mc, nullptr, e->d_twiddle);
   const int fft_d4c = (int)pow(2.0, 1.0 + (int)(log(4.0 * fs / 47.0 + 1) / kLog2));   // host pow: exact
   const int lt_fft = (int)pow(2.0, 1.0 + (int)(log(3.0 * fs / 40.0 + 1) / kLog2));
+#ifdef RYK_D4C_TIMELINE
+  { unsigned long long* tl_ = nullptr; cudaGetSymbolAddress((void**)&tl_, g_d4c_tl); cudaMemsetAsync(tl_, 0, sizeof(g_d4c_tl), st); }
+#endif
   k_d4c<<<n_out, 512, d4c_smem_bytes(fs), st>>>(d_x, n, fs, frame_period, d_f0, fft_size, 0.85, n_out, d_ap, e->d_twiddle, fft_d4c, lt_fft);
+#ifdef RYK_D4C_TIMELINE
+  cudaStreamCaptureStatus cap_ = cudaStreamCaptureStatusNone;
+  cudaStreamIsCapturing(st, &cap_);
+  if (const char* path = cap_ == cudaStreamCaptureStatusNone ? getenv("RYK_D4C_TIMELINE_FILE") : nullptr) {
+    cudaStreamSynchronize(st);
+    static std::vector<unsigned long long> h(kD4cTlMaxCtas * kD4cTlSlots);
+    cudaMemcpyFromSymbol(h.data(), g_d4c_tl, sizeof(unsigned long long) * h.size());
+    if (FILE* f = fopen(path, "a")) {
+      fprintf(f, "# launch: %d frames, slots 0..%d\n", n_out, kD4cTlSlots - 1);
+      for (int c = 0; c < n_out && c < kD4cTlMaxCtas; ++c) { for (int k = 0; k < kD4cTlSlots; ++k) fprintf(f, "%llu ", h[c * kD4cTlSlots + k]); fprintf(f, "\n"); }
+      fclose(f);
+    }
+  }
+#endif
   k_f0_out<<<(n_out + 127) / 128, 128, 0, st>>>(d_f0, n_out, d_f0_out, d_voiced);
   RYK_CUDA(cudaGetLastError());
   return 0;

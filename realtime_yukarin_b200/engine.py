@@ -52,7 +52,7 @@ EXPORTED_SYMBOLS = [
     'ryk_stage2_convert', 'ryk_convert_window', 'ryk_synth_create', 'ryk_synth_destroy', 'ryk_synth_add_parameters',
     'ryk_synth_synthesis2', 'ryk_synth_decode', 'ryk_session_create', 'ryk_session_destroy', 'ryk_session_push',
     'ryk_session_push_device', 'ryk_session_submit', 'ryk_session_collect', 'ryk_group_create', 'ryk_group_destroy',
-    'ryk_group_size', 'ryk_session_stage_times', 'ryk_group_submit', 'ryk_group_collect', 'ryk_group_push_device', 'ryk_test_conv_layer', 'ryk_debug_dio', 'ryk_debug_synth_pulses', 'ryk_debug_synth_timebase', 'ryk_engine_profile', 'ryk_engine_profile_read', 'ryk_engine_timer_start', 'ryk_engine_timer_stop',
+    'ryk_group_size', 'ryk_session_stage_times', 'ryk_group_submit', 'ryk_group_collect', 'ryk_group_push_device', 'ryk_test_conv_layer', 'ryk_debug_dio', 'ryk_debug_stonemask', 'ryk_debug_synth_pulses', 'ryk_debug_synth_timebase', 'ryk_engine_profile', 'ryk_engine_profile_read', 'ryk_engine_timer_start', 'ryk_engine_timer_stop',
     'ryk_world_synthesize_length', 'ryk_world_synthesize', 'ryk_output_gate', 'ryk_reblock_create', 'ryk_reblock_destroy',
     'ryk_reblock_push', 'ryk_reblock_push_device', 'ryk_reblock_collect', 'ryk_reblock_result_device', 'ryk_resample_length',
     'ryk_resample_poly', 'ryk_session_poll', 'ryk_reblock_poll', 'ryk_engine_profile_read2', 'ryk_engine_set_stage1_fused',
@@ -439,6 +439,15 @@ class Engine(object):
         self._check(self.lib.ryk_debug_dio(self._h, int(n), int(fs), ctypes.c_double(frame_period), ctypes.c_double(f0_floor),
                                            ctypes.c_double(f0_ceil), _dp(f0), _dp(cand), _dp(score), counts.ctypes.data_as(c_int_p)))
         return f0, cand, score, counts
+
+    def debug_stonemask(self, x, fs, frame_period, f0_floor, f0_in):
+        """StoneMask alone on the given f0 estimates (one per frame), shared memory sized from f0_floor as in analysis."""
+        x = _f32(x)
+        f0_in = numpy.ascontiguousarray(f0_in, dtype=numpy.float64)
+        f0 = numpy.empty(len(f0_in))
+        self._check(self.lib.ryk_debug_stonemask(self._h, _fp(x), len(x), int(fs), ctypes.c_double(frame_period),
+                                                 ctypes.c_double(f0_floor), _dp(f0_in), len(f0_in), _dp(f0)))
+        return f0
 
     def test_conv_layer(self, in0, in1, W, scale, shift, transposed, k, stride, pad, act, use_tc, repeat=0):
         """One conv layer in isolation; in0/in1 NHWC float32, W in the Chainer layout. Returns (out NHWC, ms per run)."""
